@@ -4,8 +4,10 @@
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload antmaze-large] [--batch 256] [--seeds 1]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...     (N > 1, one rank per GPU)
   python bench.py --impl reference ...       CPU arm: the oracle's fp32 restatement of the reference on the host cores
+  python bench.py ... --dump-outputs DIR     also write the metrics and parameters of the last timed step as DIR/<name>.npy
 
-A "step" is one FQLAgent.update (agents/fql.py:122-133) on one synthetic batch of the named OGBench shape.
+A "step" is one FQLAgent.update (agents/fql.py:122-133) on one synthetic batch of the named OGBench shape.  The K timed steps are
+steps W+1 .. W+K of one training run from the seeded initial state, so with the same arguments every run computes the same outputs.
   value   device-timed samples/s with the batch already resident in HBM (CUDA events around every step, max over ranks)
   e2e     the same through the public API `agent.update(host_batch)`: pinned H2D of the batch + D2H of the 13 metrics
 N > 1 is data parallel, weak scaling: every rank holds `--batch` rows of a global batch of N*batch; the gradient buckets are
@@ -168,7 +170,7 @@ def cpu_reference_arm(wl, B, steps, warmup, budget_s=20.0):
         t0 = time.perf_counter()
         info, _ = agent.update(batches[i % 4], noises[i % 4])
         times.append(time.perf_counter() - t0)
-        if time.perf_counter() - t_begin > budget_s and len(times) >= 3:
+        if budget_s is not None and time.perf_counter() - t_begin > budget_s and len(times) >= 3:
             break
     times.sort()
     med = times[len(times) // 2]
@@ -254,6 +256,22 @@ def euler_kernel_traffic_from_profile():
     return None, None
 
 
+def write_outputs(out_dir, arrays, limit=64 * 10 ** 6):
+    """--dump-outputs: one float32 DIR/<name>.npy per array.  Past `limit` bytes in all, every array of more than 4096 elements is cut
+    to the same fraction of its flattened elements, picked with a fixed seed, so two runs with the same arguments still compare
+    element for element."""
+    import numpy as np
+    arrays = {k: np.asarray(v, np.float32) for k, v in arrays.items()}
+    small = sum(a.size for a in arrays.values() if a.size <= 4096) * 4
+    big = sum(a.size for a in arrays.values() if a.size > 4096) * 4
+    frac = min(1.0, (limit - small - 256 * len(arrays)) / max(big, 1))    # 256 bytes: room for each .npy header
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if frac < 1.0 and a.size > 4096:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, int(a.size * frac), replace=False))]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -268,7 +286,14 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-fp32-leg', action='store_true')
     ap.add_argument('--no-scaling-configs', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the metrics and the parameters of the last timed step as DIR/<name>.npy (float32, at most 64 MB '
+                         'in all: larger parameter sets are written as a fixed, seeded sample)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes what the b200 implementation computed')
     wl = WORKLOADS[args.workload]
     # pixel workloads: --precision bf16 = the ImpalaEncoders on tcgen05 in bf16 (FQL_PRECISION_BF16_ENC), MLPs behind them in fp32
     F, A = wl['F'], wl['A']
@@ -283,7 +308,7 @@ def main():
     if args.impl == 'reference':
         if rank != 0:
             return 0
-        r = cpu_reference_arm(wl, args.batch, args.steps, args.warmup)
+        r = cpu_reference_arm(wl, args.batch, args.steps, args.warmup, budget_s=None)
         sps = 1e3 / r['ms_per_step']
         val = sps * args.batch
         sample = f"{r['steps_measured']} full updates of the same workload at batch {args.batch} (median), fp32 torch-CPU (MKL, autograd)"
@@ -332,6 +357,8 @@ def main():
         clocks = ClockSampler(local_rank) if rank == 0 else None
         for _ in range(W):
             agent.step(bufs)
+        # the timed steps continue from this state: the load below runs a number of steps that depends on the clock
+        warm_state = agent.state_dict()
         # keep the GPU under the same load until nvidia-smi is sampling (~0.5 s): the step count must be IDENTICAL on every rank
         # (each step contains collectives), so it is derived from a max-reduced timing, never from a per-rank clock
         torch.cuda.synchronize()
@@ -345,6 +372,7 @@ def main():
         for _ in range(int(min(3000, max(0, 0.5 / max(float(per.item()), 1e-6))))):
             agent.step(bufs)
         barrier()
+        agent.load_state_dict(warm_state)
         l0 = agent.launch_count()
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
         barrier()
@@ -356,6 +384,10 @@ def main():
         barrier()
         launches = agent.launch_count() - l0
         dev_ms = sum(a.elapsed_time(b) for a, b in ev)
+        if args.dump_outputs and rank == 0:
+            from oracle.fql_oracle import tree_leaves
+            outputs = {'info.' + k.replace('/', '.'): v for k, v in info.items()}
+            outputs.update(('params.' + '.'.join(path), v) for path, v in tree_leaves(agent.export_tree('params')))
         last_loss = float(np.ravel(info['critic/critic_loss'])[0])
         assert np.isfinite(last_loss), 'non-finite loss in the timed region'
         # L2-warm variant (no flush), reported beside the headline
@@ -517,6 +549,8 @@ def main():
         out['cpu_baseline'] = dict(value=cv, unit='samples/s', steps_per_sec=1e3 / r['ms_per_step'], cores=r['cores'], kind='port',
                                    sample=f"{r['steps_measured']} full updates at batch {args.batch}, 1 seed (median), fp32 torch-CPU "
                                           f"restatement of the reference (JAX not installable)")
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     print(json.dumps(out), flush=True)
     if world > 1:
         _shutdown(agent)

@@ -1,10 +1,11 @@
-"""Pins the oracle to the REAL reference the first time a box has jax + flax + optax + ml_collections and the reference checkout:
-imports /root/reference/agents/fql.py unmodified, loads the oracle's parameters into its TrainState, reproduces the five noise
-draws of one update with the reference's own key derivation (agents/fql.py:100,24,143,49,62,82 -- SURVEY 8a "RNG derivation"),
-and compares losses, gradients and the updated parameters of `agent.update(batch)` with oracle/fql_oracle.py on the same inputs.
+"""Pins the oracle to the REAL reference on a machine with jax + flax + optax + ml_collections and a checkout of the reference FQL
+implementation named by FQL_REFERENCE_PATH: imports $FQL_REFERENCE_PATH/agents/fql.py unmodified, loads the oracle's parameters into
+its TrainState, reproduces the five noise draws of one update with the reference's own key derivation (agents/fql.py:100,24,143,49,62,82
+-- SURVEY 8a "RNG derivation"), and compares losses, gradients and the updated parameters of `agent.update(batch)` with
+oracle/fql_oracle.py on the same inputs.
 
-In this image none of the four packages is installed (and there is no network), so the test SKIPS here: the oracle stays
-"parity unpinned" (DESIGN.md section 2) until this test has run green somewhere."""
+Without those packages or that checkout the test SKIPS: the oracle stays "parity unpinned" (DESIGN.md section 2) until this test has
+run green somewhere."""
 import copy
 import os
 import sys
@@ -17,9 +18,9 @@ pytest.importorskip('flax')
 pytest.importorskip('optax')
 pytest.importorskip('ml_collections')
 
-REF = os.environ.get('FQL_REFERENCE_PATH', '/root/reference')
-if not os.path.isfile(os.path.join(REF, 'agents', 'fql.py')):
-    pytest.skip(f'reference checkout not found at {REF}', allow_module_level=True)
+REF = os.environ.get('FQL_REFERENCE_PATH', '')
+if not REF or not os.path.isfile(os.path.join(REF, 'agents', 'fql.py')):
+    pytest.skip('FQL_REFERENCE_PATH does not name a checkout of the reference FQL implementation', allow_module_level=True)
 
 from oracle import fql_oracle as O  # noqa: E402
 from tests.helpers import make_case, rel_err  # noqa: E402
