@@ -51,6 +51,27 @@ class FqlDpComm(C.Structure):
     _fields_ = [('rank', C.c_int32), ('world', C.c_int32), ('base', C.c_void_p * DP_MAX_RANKS), ('base_mc', C.c_void_p)]
 
 
+class FqlTestOperand(C.Structure):
+    _fields_ = [('ptr', C.c_void_p), ('inner', C.c_int32), ('rows', C.c_int32), ('ld', C.c_int64), ('g0', C.c_int32), ('s0', C.c_int64),
+                ('g1', C.c_int32), ('s1', C.c_int64)]
+
+
+class FqlTestPtr(C.Structure):
+    _fields_ = [('base', C.c_void_p), ('s0', C.c_int64), ('s1', C.c_int64), ('ld', C.c_int32)]
+
+
+TEST_GEMM_PTRS = ('bias', 'out_f', 'out_h', 'out_z', 'zin', 'act', 'xb', 'target', 'ln_s', 'ln_b', 'dbias', 'wmaster', 'dln_s', 'dln_b')
+
+
+class FqlTestGemm(C.Structure):
+    _fields_ = ([(n, C.c_int32) for n in ('mode', 'M', 'N', 'K', 'G0', 'G1', 'a_mn', 'b_mn', 'ksplit')] +
+                [('A', FqlTestOperand), ('B', FqlTestOperand)] + [(n, FqlTestPtr) for n in TEST_GEMM_PTRS] +
+                [(n, C.c_int32) for n in ('F', 'Adim', 'step', 'n_steps', 'clip')])
+
+
+TC_MODE_STORE_F32, TC_MODE_FWD_HIDDEN, TC_MODE_DGRAD_GELU, TC_MODE_EULER, TC_MODE_WGRAD_LN = 0, 1, 2, 3, 4
+
+
 class FqlError(RuntimeError):
     pass
 
@@ -85,7 +106,16 @@ _SIGS = {
                                    C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     'fql_conv3x3_wgrad_bf16': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
                                          C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
-    'fql_set_early_grads_event': (C.c_int, [C.c_void_p, C.c_void_p]),
+    'fql_test_tc_gemm': (C.c_int, [C.POINTER(FqlTestGemm), C.c_void_p]),
+    'fql_test_act_ln_bf16': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    'fql_test_ln_bwd_bf16': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32,
+                                       C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_void_p]),
+    'fql_test_gelu_bwd_bf16': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                         C.c_int64, C.c_int64, C.c_void_p]),
+    'fql_test_colsum_bf16': (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_int64,
+                                       C.c_void_p]),
+    'fql_set_early_grads_event':(C.c_int, [C.c_void_p, C.c_void_p]),
     'fql_early_grads_floats': (C.c_int64, [C.POINTER(FqlDims)]),
     'fql_total_loss': (C.c_int, [C.c_void_p, C.POINTER(FqlDims), C.POINTER(FqlHparams), C.POINTER(FqlBatch), C.POINTER(FqlState),
                                  C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -779,3 +779,67 @@ extern "C" int fql_debug_tc_gemm(const void* X, const void* W, const float* bias
   g.dbg = dbg;
   return tc_gemm(g, reinterpret_cast<cudaStream_t>(stream));
 }
+
+// ---------------------------------------------------------------------------------------------------------------
+// Test hooks (include/fql_b200.h): one tc_gemm or one row / column kernel on caller buffers, with the argument meaning the step
+// uses, so that each kernel can be checked on its own against a reference.  tc_gemm's own FQL_REQUIRE checks are the validation.
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+TcOperand test_op(const FqlTestOperand& o) { return op(o.ptr, o.inner, o.rows, o.ld, o.g0, o.s0, o.g1, o.s1); }
+TcPtr test_ptr(const FqlTestPtr& p) { return tp(p.base, p.s0, p.s1, p.ld); }
+}  // namespace
+
+extern "C" int fql_test_tc_gemm(const FqlTestGemm* t, void* stream) {
+  FQL_REQUIRE(t != nullptr, "fql_test_tc_gemm: spec is NULL");
+  TcGemmSpec g;
+  memset(&g, 0, sizeof(g));
+  g.mode = t->mode; g.M = t->M; g.N = t->N; g.K = t->K; g.G0 = t->G0; g.G1 = t->G1; g.a_mn = t->a_mn; g.b_mn = t->b_mn;
+  g.ksplit = t->ksplit;
+  g.A = test_op(t->A); g.B = test_op(t->B);
+  g.bias = test_ptr(t->bias); g.out_f = test_ptr(t->out_f); g.out_h = test_ptr(t->out_h); g.out_z = test_ptr(t->out_z);
+  g.zin = test_ptr(t->zin); g.act = test_ptr(t->act); g.xb = test_ptr(t->xb); g.target = test_ptr(t->target);
+  g.ln_s = test_ptr(t->ln_s); g.ln_b = test_ptr(t->ln_b); g.dbias = test_ptr(t->dbias); g.wmaster = test_ptr(t->wmaster);
+  g.dln_s = test_ptr(t->dln_s); g.dln_b = test_ptr(t->dln_b);
+  g.F = t->F; g.Adim = t->Adim; g.step = t->step; g.n_steps = t->n_steps; g.clip = t->clip;
+  return tc_gemm(g, reinterpret_cast<cudaStream_t>(stream));
+}
+
+// rows = S * E * M, one warp per row (tc_critic_forward / tc_critic_backward launch them the same way)
+extern "C" int fql_test_act_ln_bf16(const float* Z, const float* scale, const float* bias, int64_t par_s, int64_t par_e, void* Hb, float* mu,
+                                    float* rstd, int32_t M, int32_t N, int32_t S, int32_t E, int32_t ln, void* stream) {
+  FQL_REQUIRE(M >= 1 && S >= 1 && E >= 1 && N >= 4 && N <= 128 * ROW_V && N % 4 == 0, "fql_test_act_ln_bf16: M=%d N=%d S=%d E=%d", M, N, S, E);
+  FQL_REQUIRE(!ln || (scale && bias), "fql_test_act_ln_bf16: LayerNorm needs scale and bias");
+  const int64_t rows = (int64_t)S * E * M;
+  FQL_CHECK_CUDA(fql_launch_pdl(act_ln_bf16_kernel, dim3((unsigned)((rows + ROW_WARPS - 1) / ROW_WARPS)), dim3(32 * ROW_WARPS), 0,
+                                reinterpret_cast<cudaStream_t>(stream), Z, scale, bias, par_s, par_e, reinterpret_cast<bf16*>(Hb), mu, rstd, M,
+                                N, S, E, ln));
+  FQL_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int fql_test_ln_bwd_bf16(const float* dH, const float* Z, const float* scale, int64_t scale_s, int64_t scale_e, float* dZ, void* dZb,
+                                    int32_t M, int32_t N, int32_t S, int32_t E, int64_t z_rows_e, int64_t z_rows_s, void* stream) {
+  FQL_REQUIRE(M >= 1 && S >= 1 && E >= 1 && N >= 4 && N <= 128 * ROW_V && N % 4 == 0, "fql_test_ln_bwd_bf16: M=%d N=%d S=%d E=%d", M, N, S, E);
+  const int64_t rows = (int64_t)S * E * M;
+  FQL_CHECK_CUDA(fql_launch_pdl(ln_bwd_bf16_kernel, dim3((unsigned)((rows + ROW_WARPS - 1) / ROW_WARPS)), dim3(32 * ROW_WARPS), 0,
+                                reinterpret_cast<cudaStream_t>(stream), dH, Z, scale, scale_s, scale_e, dZ, reinterpret_cast<bf16*>(dZb), M, N, S,
+                                E, z_rows_e, z_rows_s));
+  FQL_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int fql_test_gelu_bwd_bf16(const float* dH, const float* Z, float* dZ, void* dZb, int32_t M, int32_t N, int32_t S, int32_t E,
+                                      int64_t z_rows_e, int64_t z_rows_s, void* stream) {
+  FQL_REQUIRE(M >= 1 && S >= 1 && E >= 1 && N >= 1, "fql_test_gelu_bwd_bf16: M=%d N=%d S=%d E=%d", M, N, S, E);
+  const int64_t n = (int64_t)S * E * M * N;
+  FQL_CHECK_CUDA(fql_launch_pdl(gelu_bwd_bf16_kernel, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, reinterpret_cast<cudaStream_t>(stream), dH, Z,
+                                dZ, reinterpret_cast<bf16*>(dZb), M, N, S, E, z_rows_e, z_rows_s));
+  FQL_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int fql_test_colsum_bf16(const void* X, int64_t G, int64_t M, int32_t N, float* out, int64_t out_stride_g0, int32_t G0,
+                                    int64_t out_stride_g1, void* stream) {
+  FQL_REQUIRE(G0 >= 1 && G % G0 == 0, "fql_test_colsum_bf16: G=%lld G0=%d", (long long)G, G0);
+  return launch_colsum_bf16(X, G, M, N, out, out_stride_g0, G0, out_stride_g1, reinterpret_cast<cudaStream_t>(stream));
+}

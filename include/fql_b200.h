@@ -233,6 +233,43 @@ int fql_conv3x3_bf16(const void* x, const float* w_hwio, const float* bias, int3
 int fql_conv3x3_wgrad_bf16(const void* x, const void* dy, int32_t B, int32_t H, int32_t W, int32_t cin, int32_t cout, float* gw, float* gb,
                            void* workspace, size_t ws_bytes, void* stream);
 
+/* ---- test hooks: the tensor-core MLP kernels of FQL_PRECISION_BF16_TC one at a time on caller buffers ---------------------------
+ * Not used by the step; they exist so that each kernel can be compared with a reference on its own.  The arguments mean what they
+ * mean inside the step (fql_b200/csrc/step.cuh: TcGemmSpec, and the row / column kernels of tc_path.cu); enqueue-only. */
+typedef struct FqlTestOperand { /* bf16 TMA operand [g1][g0][rows][inner], pitches ld / s0 / s1 in elements */
+  const void* ptr;
+  int32_t inner, rows;
+  int64_t ld;
+  int32_t g0;
+  int64_t s0;
+  int32_t g1;
+  int64_t s1;
+} FqlTestOperand;
+typedef struct FqlTestPtr {     /* epilogue tensor at base + g0 * s0 + g1 * s1 (elements of its own type), row pitch ld */
+  void* base;
+  int64_t s0, s1;
+  int32_t ld;
+} FqlTestPtr;
+typedef struct FqlTestGemm {    /* D[M,N] = A[M,K] B[K,N] over G1 x G0 groups with the epilogue `mode` (TC_MODE_*) */
+  int32_t mode, M, N, K, G0, G1, a_mn, b_mn, ksplit;
+  FqlTestOperand A, B;
+  FqlTestPtr bias, out_f, out_h, out_z, zin, act, xb, target, ln_s, ln_b, dbias, wmaster, dln_s, dln_b;
+  int32_t F, Adim, step, n_steps, clip;
+} FqlTestGemm;
+int fql_test_tc_gemm(const FqlTestGemm* g, void* stream);
+/* H = [LayerNorm](gelu(Z)) -> bf16 (+ mu / rstd when ln); Z fp32 [S][E][M][N] dense, scale / bias at s * par_s + e * par_e */
+int fql_test_act_ln_bf16(const float* Z, const float* scale, const float* bias, int64_t par_s, int64_t par_e, void* Hb, float* mu,
+                         float* rstd, int32_t M, int32_t N, int32_t S, int32_t E, int32_t ln, void* stream);
+/* dZ = LayerNorm_bwd(dH; gelu(Z)) * gelu'(Z) (fp32 + bf16 copy); row r of group (s, e) of Z at (s * z_rows_s + e * z_rows_e + r) * N */
+int fql_test_ln_bwd_bf16(const float* dH, const float* Z, const float* scale, int64_t scale_s, int64_t scale_e, float* dZ, void* dZb,
+                         int32_t M, int32_t N, int32_t S, int32_t E, int64_t z_rows_e, int64_t z_rows_s, void* stream);
+/* dZ = dH * gelu'(Z) (fp32 + bf16 copy), Z addressed as above */
+int fql_test_gelu_bwd_bf16(const float* dH, const float* Z, float* dZ, void* dZb, int32_t M, int32_t N, int32_t S, int32_t E,
+                           int64_t z_rows_e, int64_t z_rows_s, void* stream);
+/* column sums of bf16 X [G][M][N] (N % 64 == 0) ADDED into out[g0 * out_stride_g0 + g1 * out_stride_g1 + n], g = g1 * G0 + g0 */
+int fql_test_colsum_bf16(const void* X, int64_t G, int64_t M, int32_t N, float* out, int64_t out_stride_g0, int32_t G0,
+                         int64_t out_stride_g1, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

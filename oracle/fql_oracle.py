@@ -98,14 +98,16 @@ def n_dense(p):
     return sum(1 for k in p if k.startswith('Dense_'))
 
 
-def mlp_forward(p, x, layer_norm, save=False):
+def mlp_forward(p, x, layer_norm, save=False, q=None):
+    """q: optional storage rounding of the contraction operands (e.g. to bf16), applied to every kernel and to every layer's
+    input; the bias, the pre-activations and everything after them stay in the array dtype.  None (the default) rounds nothing."""
     n = n_dense(p)
     ens = p['Dense_0']['kernel'].ndim == 3
     cache = []
     h = x
     for i in range(n):
         W, b = p[f'Dense_{i}']['kernel'], p[f'Dense_{i}']['bias']
-        z = np.matmul(h, W) + (b[:, None, :] if ens else b)
+        z = (np.matmul(h, W) if q is None else np.matmul(q(h), q(W))) + (b[:, None, :] if ens else b)
         if i + 1 < n:
             g = gelu_tanh(z)
             if layer_norm:
@@ -164,11 +166,11 @@ def mlp_backward(p, cache, dout, layer_norm, need_dx=True, need_dw=True):
 # --------------------------------------------------------------------------------------
 # modules
 # --------------------------------------------------------------------------------------
-def actor_forward(net_p, cfg, obs, actions, times=None, save=False):
+def actor_forward(net_p, cfg, obs, actions, times=None, save=False, q=None):
     """ActorVectorField.__call__ (utils/networks.py:216-235), state-based (no encoder)."""
     parts = [obs, actions] if times is None else [obs, actions, times]
     x = np.concatenate(parts, axis=-1)
-    return mlp_forward(net_p['mlp'], x, cfg['actor_layer_norm'], save=save)
+    return mlp_forward(net_p['mlp'], x, cfg['actor_layer_norm'], save=save, q=q)
 
 
 def critic_forward(net_p, cfg, obs, actions, save=False):
@@ -180,20 +182,21 @@ def critic_forward(net_p, cfg, obs, actions, save=False):
     return r[..., 0]
 
 
-def sample_actions_given_noise(params, cfg, obs, noise):
-    """agents/fql.py:135-153 with the noise draw made explicit."""
-    a = actor_forward(params['modules_actor_onestep_flow'], cfg, obs, noise)
+def sample_actions_given_noise(params, cfg, obs, noise, q=None):
+    """agents/fql.py:135-153 with the noise draw made explicit (q: see mlp_forward)."""
+    a = actor_forward(params['modules_actor_onestep_flow'], cfg, obs, noise, q=q)
     return np.clip(a, -1, 1)
 
 
-def compute_flow_actions(params, cfg, obs, noises):
-    """agents/fql.py:155-171."""
+def compute_flow_actions(params, cfg, obs, noises, q=None):
+    """agents/fql.py:155-171.  q (see mlp_forward) rounds each step's network input, so the velocity field sees the rounded copy of
+    the actions and of the time while the Euler state itself keeps the array dtype."""
     dt = obs.dtype.type
     n = cfg['flow_steps']
     a = noises
     for i in range(n):
         t = np.full(obs.shape[:-1] + (1,), i / n, dtype=obs.dtype)  # python float -> array dtype (fql.py:167)
-        v = actor_forward(params['modules_actor_bc_flow'], cfg, obs, a, t)
+        v = actor_forward(params['modules_actor_bc_flow'], cfg, obs, a, t, q=q)
         a = a + v / dt(n)
     return np.clip(a, -1, 1)
 
