@@ -31,8 +31,6 @@
 #include "step.cuh"
 #include "tc_prims.cuh"
 
-#include <cudaTypedefs.h>
-
 using namespace tc;
 
 namespace {
@@ -142,13 +140,7 @@ __device__ __forceinline__ float bf16_at(const uint4 (&q)[4], int i) {
   return __uint_as_float((i & 1) ? (w & 0xffff0000u) : (w << 16));
 }
 
-// PAIR: two CTAs of a 2-CTA cluster (consecutive 128-row tiles of one group) run as a cta_group::2 pair: ONE tcgen05.mma issued by the
-// leader covers both tiles (M = 256), each CTA holds half of every weight stage (its 128 of the 256 columns of an N-half) and its own
-// activations / accumulator rows / epilogue.  The serial work of the single MMA-issuing thread bounds this kernel (profiles/r2f_chain2_*): the pair does
-// the same number of tcgen05.mma / tcgen05.commit per 256 rows that one CTA needs per 128.  Barriers the leader's MMA thread waits on
-// (full, a_ready, acc_free, x_full, x_ready) live in the leader and take the peer's arrivals remotely; barriers the epilogue / producer
-// warps wait on (empty, a_free, acc_full) are signalled in both CTAs by multicast tcgen05.commit.
-template <int MODE, bool PAIR>
+template <int MODE>
 __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_constant__ CUtensorMap mapX,
                                                               const __grid_constant__ CUtensorMap mapW,
                                                               const __grid_constant__ CUtensorMap mapWL,
@@ -157,16 +149,13 @@ __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_
   constexpr bool BWD = (MODE == C2_BWD || MODE == C2_BWD_LN);
   constexpr bool EULER = (MODE == C2_EULER);
   constexpr int NPAR = BWD ? (LN ? 1 : 0) : (LN ? 3 : 1);
-  constexpr int NCTA = PAIR ? 2 : 1;
-  constexpr int SLOT = STAGE_BYTES / NCTA;              // a CTA's part of one weight stage
-  const uint32_t rank = PAIR ? cluster_ctarank_() : 0u; // 0 = leader
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   const int nkb_x = BWD ? 1 : a.K0pad / 64;
   uint8_t* sA = smem;                                   // [8][16 KB]
   uint8_t* sX = sA + NKB * KB_BYTES;                    // [nkb_x][16 KB]
   uint8_t* sW = sX + nkb_x * KB_BYTES;                  // [nstage][16 KB]
-  float* sPar = reinterpret_cast<float*>(sW + a.nstage * SLOT);  // [2][NPAR][512]: bias (, LN scale, LN bias) / LN scale
+  float* sPar = reinterpret_cast<float*>(sW + a.nstage * STAGE_BYTES);  // [2][NPAR][512]: bias (, LN scale, LN bias) / LN scale
   float* sStat = sPar + 2 * NPAR * HID;                 // [2][128][2] row sums of the two column parities (LayerNorm)
   uint64_t* bars = reinterpret_cast<uint64_t*>(sStat + (LN ? 2 * TILE_M * 2 : 0));
   uint64_t* full = bars;                 // [8]
@@ -196,54 +185,41 @@ __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_
     for (int i = 0; i < 8; i++) {
       mbar_init(&full[i], 1);
       mbar_init(&empty[i], 1);
-      mbar_init(&a_ready[i], EPI_WARPS * NCTA);
+      mbar_init(&a_ready[i], EPI_WARPS);
     }
     for (int i = 0; i < 4; i++) mbar_init(&a_free[i], 1);
     for (int i = 0; i < 2; i++) {
       mbar_init(&acc_full[i], 1);
-      mbar_init(&acc_free[i], EPI_WARPS * NCTA);
+      mbar_init(&acc_free[i], EPI_WARPS);
     }
     mbar_init(x_full, 1);
-    mbar_init(x_ready, EPI_WARPS * NCTA);
+    mbar_init(x_ready, EPI_WARPS);
     fence_barrier_init();
   }
-  if (warp == 1) {
-    if (PAIR) tmem_alloc2(tmem_slot, 512);
-    else tmem_alloc(tmem_slot, 512);
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, 512);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  if (PAIR) cluster_sync_();     // both CTAs' barriers are initialised before any remote arrive / completion
   const uint32_t tmem_base = *tmem_slot;
   // The TMA producer and the MMA issuer are ONE thread each, but all 32 lanes of their warps run the loops (waits, descriptor arithmetic):
   // warp-uniform control flow keeps the descriptors in uniform registers, and only the instruction itself is predicated on the elected
   // lane.  With the whole loop under `if (lane == 0)` ptxas wraps every tcgen05.mma / tcgen05.commit / TMA in an ELECT + 5 R2UR.BROADCAST
   // waterfall: 178 instead of 139 ns per two MMAs + commit in isolation (profiles/micro/mma_dual_bench.cu), 370 ns per stage in here.
   bool el = false;     // set at the top of the two roles' branches (straight from elect.sync: ptxas then knows the region is single-lane)
-  // arrive on a barrier the leader's MMA thread waits on
-  auto arrive_lead = [&](uint64_t* bar) {
-    if (!PAIR || rank == 0) mbar_arrive(bar);
-    else mbar_arrive_remote(bar, 0);
-  };
-  // wait on a barrier that takes arrivals from the peer CTA (remote arrive / multicast commit / the peer's TMA)
+  // the producer and the issuer spin with the wait loop inside the asm block (see mbar_wait_u)
   auto wait_x = [&](uint64_t* bar, uint32_t parity) {
-    if (PAIR) mbar_wait_cl(bar, parity);
-    else if (warp <= 1) mbar_wait_u(bar, parity);
+    if (warp <= 1) mbar_wait_u(bar, parity);
     else mbar_wait(bar, parity);
   };
-  // TMA load of this CTA's part of a stage; completion bytes go to the leader's barrier
   auto load2d = [&](void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1) {
-    if (!el) return;
-    if (PAIR && rank != 0) tma_load_2d_pair(dst, m, bar, c0, c1);
-    else tma_load_2d(dst, m, bar, c0, c1);
+    if (el) tma_load_2d(dst, m, bar, c0, c1);
   };
 
   if (warp == 0) {
     // ================= TMA producer =================
     el = elect_one();
     {
-      if (el && rank == 0) mbar_expect_tx(x_full, NCTA * nkb_x * KB_BYTES);
+      if (el) mbar_expect_tx(x_full, nkb_x * KB_BYTES);
       const int xrow = a.x_row0[p] + s * a.x_rows_s + e * a.x_rows_e + tile * TILE_M;
       for (int kb = 0; kb < nkb_x; kb++) load2d(sX + kb * KB_BYTES, &mapX, x_full, kb * 64, xrow);
       int stage = 0;
@@ -261,15 +237,15 @@ __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_
             for (int ks = 0; ks < nst; ks++) {
               wait_x(&empty[stage], phase ^ 1);
               C2_STAMP(n == FQL_C2_DBG_N && MODE == C2_EULER, 128 + h * 16 + ks);
-              uint8_t* dst = sW + stage * SLOT;
-              if (el && rank == 0) mbar_expect_tx(&full[stage], STAGE_BYTES);
-              if (BWD) {     // this CTA's 256 / NCTA input rows of the half
-                load2d(dst, it == 0 ? &mapWL : &mapW, &full[stage], ks * KS, row0 + h * NHALF + (int)rank * (NHALF / NCTA));
-              } else if (!PAIR && a.w3d) {
+              uint8_t* dst = sW + stage * STAGE_BYTES;
+              if (el) mbar_expect_tx(&full[stage], STAGE_BYTES);
+              if (BWD) {     // the 256 input rows of the half
+                load2d(dst, it == 0 ? &mapWL : &mapW, &full[stage], ks * KS, row0 + h * NHALF);
+              } else if (a.w3d) {
                 if (el) tma_load_3d(dst, &mapW, &full[stage], 0, row0 + ks * KS, h * 4);
-              } else {       // this CTA's 4 / NCTA chunks of 64 output columns of the half
-                for (int c = 0; c < 4 / NCTA; c++)
-                  load2d(dst + c * CHUNK_BYTES, &mapW, &full[stage], (h * 4 + (int)rank * (4 / NCTA) + c) * 64, row0 + ks * KS);
+              } else {       // the 4 chunks of 64 output columns of the half
+                for (int c = 0; c < 4; c++)
+                  load2d(dst + c * CHUNK_BYTES, &mapW, &full[stage], (h * 4 + c) * 64, row0 + ks * KS);
               }
               if (++stage == a.nstage) { stage = 0; phase ^= 1; }
             }
@@ -278,107 +254,98 @@ __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_
           const int row0 = BWD ? a.w_row[p][0] + s * a.w_rows_s + e * a.K0 : a.wl_row[p] + s * a.wl_rows_s + e * HID;
           for (int ks = 0; ks < HID / KS; ks++) {
             wait_x(&empty[stage], phase ^ 1);
-            // backward: this CTA's K0pad / NCTA input rows; forward: the padded 64 output columns (the pair: N = 128, both CTAs load
-            // the same chunk, the leader's copy gives columns [0, 64) of every row of both tiles)
-            if (el && rank == 0) mbar_expect_tx(&full[stage], BWD ? a.K0pad * 64 : NCTA * KS * 128);
-            if (BWD) load2d(sW + stage * SLOT, &mapW0, &full[stage], ks * KS, row0 + (int)rank * (a.K0pad / NCTA));
-            else load2d(sW + stage * SLOT, &mapWL, &full[stage], 0, row0 + ks * KS);
+            // backward: the K0pad input rows; forward: the padded 64 output columns
+            if (el) mbar_expect_tx(&full[stage], BWD ? a.K0pad * 64 : KS * 128);
+            if (BWD) load2d(sW + stage * STAGE_BYTES, &mapW0, &full[stage], ks * KS, row0);
+            else load2d(sW + stage * STAGE_BYTES, &mapWL, &full[stage], 0, row0 + ks * KS);
             if (++stage == a.nstage) { stage = 0; phase ^= 1; }
           }
         }
       }
     }
   } else if (warp == 1) {
-    // ================= MMA issuer (the leader's only) =================
+    // ================= MMA issuer =================
     el = elect_one();
-    if (rank == 0) {
-      const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);   // uniform copy (the shared-memory load is per-thread to ptxas)
-      const uint32_t idesc_h = make_idesc_bf16(128 * NCTA, NHALF, false, !BWD);
-      const uint32_t idesc_t = make_idesc_bf16(128 * NCTA, (!BWD && PAIR) ? 128 : ntail, false, !BWD);
-      auto mma = [&](uint32_t d, uint64_t ad, uint64_t bd, uint32_t id, uint32_t acc) {
-        if (!el) return;
-        if (PAIR) umma2_bf16(d, ad, bd, id, acc);
-        else umma_bf16(d, ad, bd, id, acc);
-      };
-      auto mma_x2 = [&](uint32_t d, uint64_t ad, uint64_t bd, uint64_t as, uint64_t bs, uint32_t id, uint32_t acc) {
-        if (!el) return;
-        if (PAIR) umma2_bf16_x2(d, ad, bd, as, bs, id, acc);
-        else umma_bf16_x2(d, ad, bd, as, bs, id, acc);
-      };
-      auto commit = [&](uint64_t* bar) {
-        if (!el) return;
-        if (PAIR) umma2_commit(bar);
-        else umma_commit(bar);
-      };
-      const uint64_t a_t = make_smem_desc(0, 16, 1024);
-      // B: forward MN-major (64-column chunks CHUNK_BYTES apart, 8-k groups 1024 B apart); backward K-major rows of 64 B (SWIZZLE_64B)
-      const uint64_t b_t = BWD ? make_smem_desc_sw64(0, 16, 512) : make_smem_desc(0, CHUNK_BYTES, 1024);
-      const uint64_t b_k16 = BWD ? 2 : (2048 >> 4);      // second 16-k step inside a stage
-      const uint32_t sa0 = smem_u32(sA) >> 4, sx0 = smem_u32(sX) >> 4, sw0 = smem_u32(sW) >> 4;
-      int stage = 0;
-      uint32_t phase = 0;
-      int n_ar = 0, n_xr = 0;
-      int uses[2] = {0, 0};
-      int it = 0;
-      for (int n = 0; n < total; n++, it = (it + 1 == NIT) ? 0 : it + 1) {
-        if (it == 0) {
-          if (n == 0) wait_x(x_full, 0);
-          else wait_x(x_ready, (n_xr++) & 1);
-          tc_fence_after();
-        }
-        if (it < NWIDE) {
-          const int K = BWD ? (it == 0 ? 64 : HID) : (it == 0 ? a.K0 : HID);
-          const int nst = (K + KS - 1) / KS;
-          const uint32_t abase = (it == 0) ? sx0 : sa0;
-          for (int h = 0; h < 2; h++) {
-            if (uses[h] > 0) {
-              wait_x(&acc_free[h], (uses[h] - 1) & 1);
-              tc_fence_after();
-            }
-            const uint32_t tacc = tmem_u + h * NHALF;
-            for (int ks = 0; ks < nst; ks++) {
-              const int kb = ks >> 1;
-              if (it > 0 && h == 0 && (ks & 1) == 0) {
-                wait_x(&a_ready[kb], (n_ar - 1) & 1);
-                tc_fence_after();
-              }
-              C2_STAMP(n == FQL_C2_DBG_N && MODE == C2_EULER, h * 48 + ks * 3 + 0);
-              wait_x(&full[stage], phase);
-              tc_fence_after();
-              C2_STAMP(n == FQL_C2_DBG_N && MODE == C2_EULER, h * 48 + ks * 3 + 1);
-              const uint64_t adesc = a_t + (uint64_t)(abase + kb * (KB_BYTES >> 4) + (ks & 1) * 4);
-              const uint64_t bdesc = b_t + (uint64_t)(sw0 + stage * (SLOT >> 4));
-              // both K steps of a stage from ONE asm block (the second descriptor pair is a constant add inside PTX)
-              if (K - ks * KS > 16) mma_x2(tacc, adesc, bdesc, 2, b_k16, idesc_h, ks > 0);
-              else mma(tacc, adesc, bdesc, idesc_h, ks > 0);
-              commit(&empty[stage]);
-              C2_STAMP(n == FQL_C2_DBG_N && MODE == C2_EULER, h * 48 + ks * 3 + 2);
-              if (++stage == a.nstage) { stage = 0; phase ^= 1; }
-              if (it > 0 && h == 1 && (ks & 1) == 1 && kb < 4) commit(&a_free[kb]);
-            }
-            commit(&acc_full[h]);
-            uses[h]++;
-          }
-          n_ar++;
-        } else {
-          if (uses[0] > 0) {
-            wait_x(&acc_free[0], (uses[0] - 1) & 1);
+    const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);   // uniform copy (the shared-memory load is per-thread to ptxas)
+    const uint32_t idesc_h = make_idesc_bf16(TILE_M, NHALF, false, !BWD);
+    const uint32_t idesc_t = make_idesc_bf16(TILE_M, ntail, false, !BWD);
+    auto mma = [&](uint32_t d, uint64_t ad, uint64_t bd, uint32_t id, uint32_t acc) {
+      if (el) umma_bf16(d, ad, bd, id, acc);
+    };
+    auto mma_x2 = [&](uint32_t d, uint64_t ad, uint64_t bd, uint64_t as, uint64_t bs, uint32_t id, uint32_t acc) {
+      if (el) umma_bf16_x2(d, ad, bd, as, bs, id, acc);
+    };
+    auto commit = [&](uint64_t* bar) {
+      if (el) umma_commit(bar);
+    };
+    const uint64_t a_t = make_smem_desc(0, 16, 1024);
+    // B: forward MN-major (64-column chunks CHUNK_BYTES apart, 8-k groups 1024 B apart); backward K-major rows of 64 B (SWIZZLE_64B)
+    const uint64_t b_t = BWD ? make_smem_desc_sw64(0, 16, 512) : make_smem_desc(0, CHUNK_BYTES, 1024);
+    const uint64_t b_k16 = BWD ? 2 : (2048 >> 4);      // second 16-k step inside a stage
+    const uint32_t sa0 = smem_u32(sA) >> 4, sx0 = smem_u32(sX) >> 4, sw0 = smem_u32(sW) >> 4;
+    int stage = 0;
+    uint32_t phase = 0;
+    int n_ar = 0, n_xr = 0;
+    int uses[2] = {0, 0};
+    int it = 0;
+    for (int n = 0; n < total; n++, it = (it + 1 == NIT) ? 0 : it + 1) {
+      if (it == 0) {
+        if (n == 0) wait_x(x_full, 0);
+        else wait_x(x_ready, (n_xr++) & 1);
+        tc_fence_after();
+      }
+      if (it < NWIDE) {
+        const int K = BWD ? (it == 0 ? 64 : HID) : (it == 0 ? a.K0 : HID);
+        const int nst = (K + KS - 1) / KS;
+        const uint32_t abase = (it == 0) ? sx0 : sa0;
+        for (int h = 0; h < 2; h++) {
+          if (uses[h] > 0) {
+            wait_x(&acc_free[h], (uses[h] - 1) & 1);
             tc_fence_after();
           }
-          for (int ks = 0; ks < HID / KS; ks++) {
+          const uint32_t tacc = tmem_u + h * NHALF;
+          for (int ks = 0; ks < nst; ks++) {
             const int kb = ks >> 1;
-            if ((ks & 1) == 0) wait_x(&a_ready[kb], (n_ar - 1) & 1);
+            if (it > 0 && h == 0 && (ks & 1) == 0) {
+              wait_x(&a_ready[kb], (n_ar - 1) & 1);
+              tc_fence_after();
+            }
+            C2_STAMP(n == FQL_C2_DBG_N && MODE == C2_EULER, h * 48 + ks * 3 + 0);
             wait_x(&full[stage], phase);
             tc_fence_after();
-            const uint64_t adesc = a_t + (uint64_t)(sa0 + kb * (KB_BYTES >> 4) + (ks & 1) * 4);
-            const uint64_t bdesc = b_t + (uint64_t)(sw0 + stage * (SLOT >> 4));
-            mma_x2(tmem_u, adesc, bdesc, 2, b_k16, idesc_t, ks > 0);
+            C2_STAMP(n == FQL_C2_DBG_N && MODE == C2_EULER, h * 48 + ks * 3 + 1);
+            const uint64_t adesc = a_t + (uint64_t)(abase + kb * (KB_BYTES >> 4) + (ks & 1) * 4);
+            const uint64_t bdesc = b_t + (uint64_t)(sw0 + stage * (STAGE_BYTES >> 4));
+            // both K steps of a stage from ONE asm block (the second descriptor pair is a constant add inside PTX)
+            if (K - ks * KS > 16) mma_x2(tacc, adesc, bdesc, 2, b_k16, idesc_h, ks > 0);
+            else mma(tacc, adesc, bdesc, idesc_h, ks > 0);
             commit(&empty[stage]);
+            C2_STAMP(n == FQL_C2_DBG_N && MODE == C2_EULER, h * 48 + ks * 3 + 2);
             if (++stage == a.nstage) { stage = 0; phase ^= 1; }
+            if (it > 0 && h == 1 && (ks & 1) == 1 && kb < 4) commit(&a_free[kb]);
           }
-          commit(&acc_full[0]);
-          uses[0]++;
+          commit(&acc_full[h]);
+          uses[h]++;
         }
+        n_ar++;
+      } else {
+        if (uses[0] > 0) {
+          wait_x(&acc_free[0], (uses[0] - 1) & 1);
+          tc_fence_after();
+        }
+        for (int ks = 0; ks < HID / KS; ks++) {
+          const int kb = ks >> 1;
+          if ((ks & 1) == 0) wait_x(&a_ready[kb], (n_ar - 1) & 1);
+          wait_x(&full[stage], phase);
+          tc_fence_after();
+          const uint64_t adesc = a_t + (uint64_t)(sa0 + kb * (KB_BYTES >> 4) + (ks & 1) * 4);
+          const uint64_t bdesc = b_t + (uint64_t)(sw0 + stage * (STAGE_BYTES >> 4));
+          mma_x2(tmem_u, adesc, bdesc, 2, b_k16, idesc_t, ks > 0);
+          commit(&empty[stage]);
+          if (++stage == a.nstage) { stage = 0; phase ^= 1; }
+        }
+        commit(&acc_full[0]);
+        uses[0]++;
       }
     }
   } else {
@@ -461,13 +428,13 @@ __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_
               // block j >> 1 of sA still holds this layer's input until the second half's MMAs have consumed it
               if (it > 0 && h == 0) wait_x(&a_free[j >> 1], n_af & 1);
               store_chunk(sA, row, j, hv, Hb ? Hb + j * 32 : nullptr);
-              if (PAIR) fence_proxy_async_all(); else fence_proxy_async_smem();
+              fence_proxy_async_smem();
               __syncwarp();
-              if (lane == 0) arrive_lead(&a_ready[j >> 1]);
+              if (lane == 0) mbar_arrive(&a_ready[j >> 1]);
             }
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) arrive_lead(&acc_free[h]);
+            if (lane == 0) mbar_arrive(&acc_free[h]);
           }
           if (it > 0) n_af++;
         } else if (MODE == C2_BWD) {
@@ -489,13 +456,13 @@ __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_
               if (jj < 3) load_bf16x32(DGb + (j + 2) * 32, valid, dq);
               if (it > 0 && h == 0) wait_x(&a_free[j >> 1], n_af & 1);
               store_chunk(sA, row, j, hv, dZb ? dZb + j * 32 : nullptr);
-              if (PAIR) fence_proxy_async_all(); else fence_proxy_async_smem();
+              fence_proxy_async_smem();
               __syncwarp();
-              if (lane == 0) arrive_lead(&a_ready[j >> 1]);
+              if (lane == 0) mbar_arrive(&a_ready[j >> 1]);
             }
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) arrive_lead(&acc_free[h]);
+            if (lane == 0) mbar_arrive(&acc_free[h]);
           }
           if (it > 0) n_af++;
         } else if (MODE == C2_FWD_LN) {
@@ -572,13 +539,13 @@ __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_
 #pragma unroll
               for (int i = 0; i < 32; i++) hv[i] = hv[i] * par[HID + j * 32 + i] + par[2 * HID + j * 32 + i];
               store_chunk(sA, row, j, hv, Hb ? Hb + j * 32 : nullptr);
-              if (PAIR) fence_proxy_async_all(); else fence_proxy_async_smem();
+              fence_proxy_async_smem();
               __syncwarp();
-              if (lane == 0) arrive_lead(&a_ready[j >> 1]);
+              if (lane == 0) mbar_arrive(&a_ready[j >> 1]);
             }
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) arrive_lead(&acc_free[h]);
+            if (lane == 0) mbar_arrive(&acc_free[h]);
           }
         } else {  // C2_BWD_LN
           const __nv_bfloat16* XHb = reinterpret_cast<const __nv_bfloat16*>(a.XHb[l]) + rowoff;
@@ -628,13 +595,13 @@ __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_
 #pragma unroll
               for (int i = 0; i < 32; i++) hv[i] = bf16_at(dq, i) * rstd * (__uint_as_float(r[i]) - m1 - bf16_at(xq, i) * m2);
               store_chunk(sA, row, j, hv, dZb ? dZb + j * 32 : nullptr);
-              if (PAIR) fence_proxy_async_all(); else fence_proxy_async_smem();
+              fence_proxy_async_smem();
               __syncwarp();
-              if (lane == 0) arrive_lead(&a_ready[j >> 1]);
+              if (lane == 0) mbar_arrive(&a_ready[j >> 1]);
             }
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) arrive_lead(&acc_free[h]);
+            if (lane == 0) mbar_arrive(&acc_free[h]);
           }
         }
       } else {
@@ -691,23 +658,19 @@ __global__ void __launch_bounds__(C2_THREADS, 1) mlp_chain2_kernel(const __grid_
             }
           }
         }
-        if (PAIR) fence_proxy_async_all(); else fence_proxy_async_smem();
+        fence_proxy_async_smem();
         tc_fence_before();
         __syncwarp();
         if (lane == 0) {
-          arrive_lead(&acc_free[0]);
-          if (EULER) arrive_lead(x_ready);
+          mbar_arrive(&acc_free[0]);
+          if (EULER) mbar_arrive(x_ready);
         }
       }
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (PAIR) cluster_sync_();     // no CTA exits (or frees TMEM) while its peer's MMAs / arrivals can still touch it
-  if (warp == 1) {
-    if (PAIR) tmem_dealloc2(tmem_base, 512);
-    else tmem_dealloc(tmem_base, 512);
-  }
+  if (warp == 1) tmem_dealloc(tmem_base, 512);
 }
 
 #ifdef FQL_C2_DBG
@@ -718,32 +681,6 @@ extern "C" int fql_debug_chain2_stamps(unsigned long long* host_out, int n) {
 }
 namespace {
 #endif
-
-PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
-  static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-  }
-  return fn;
-}
-
-int make_map_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t rows, uint32_t box_inner, uint32_t box_rows,
-                CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B) {
-  auto enc = get_encode();
-  FQL_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is not available from the driver");
-  cuuint64_t dims[2] = {inner, rows};
-  cuuint64_t strides[1] = {inner * 2};
-  cuuint32_t box[2] = {box_inner, box_rows};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  FQL_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (%d) inner=%llu rows=%llu", (int)r, (unsigned long long)inner,
-              (unsigned long long)rows);
-  return 0;
-}
 
 // The weight matrix [rows][512] as a 3-D tensor (64 n, row, chunk of 64 n): one box {64, KS, 4} lands a whole [4][KS][64] stage.
 // The chunk dimension's stride (128 B) is smaller than the row dimension's (1024 B); returns false when the driver refuses that.
@@ -790,33 +727,19 @@ int fill_common(Chain2Args& a, const FqlDims* d, const Layout& L, int P, const i
   return 0;
 }
 
-// FQL_B200_CHAIN2_PAIR=1: CTA pairs (cta_group::2) when a group has at least two row tiles.  Parity-tested, but OFF by default: measured
-// slower (B=16384 step 2.71 vs 2.24 ms, measured before the issuer loops became warp-uniform).  The kernel is bound by the serial work of
-// its MMA-issuing thread (barrier waits, tcgen05.mma, tcgen05.commit); a pair halves the instructions per row but also halves the issuing threads per SM, so a layer of 256 rows takes 15.4 us on two
-// SMs against 12.4 us for two independent 128-row CTAs (in-kernel stamps), and the peer's remote barrier arrivals lengthen the epilogue.
-bool chain2_pair(int tiles) {
-  static const bool on = []() {
-    const char* e = getenv("FQL_B200_CHAIN2_PAIR");
-    return e && e[0] == '1';
-  }();
-  return on && tiles >= 2;
-}
-
-template <int MODE, bool PAIR>
-int launch_chain2_t(const Chain2Args& a0, int nkb_x, int npar, bool ln, const CUtensorMap& mapX, const CUtensorMap& mapW, const CUtensorMap& mapWL,
-                    const CUtensorMap& mapW0, cudaStream_t st) {
+template <int MODE>
+int launch_chain2(const Chain2Args& a0, int nkb_x, int npar, bool ln, const CUtensorMap& mapX, const CUtensorMap& mapW, const CUtensorMap& mapWL,
+                  const CUtensorMap& mapW0, cudaStream_t st) {
   Chain2Args a = a0;
-  constexpr int SLOT = STAGE_BYTES / (PAIR ? 2 : 1);
   const int fixed = (NKB + nkb_x) * KB_BYTES + 2 * npar * HID * 4 + (ln ? 2 * TILE_M * 2 * 4 : 0) + 512 + 1024;
-  int nstage = (232448 - fixed) / SLOT;
+  int nstage = (232448 - fixed) / STAGE_BYTES;
   if (nstage > 8) nstage = 8;
   static const int cap = getenv("FQL_B200_CHAIN2_STAGES") ? atoi(getenv("FQL_B200_CHAIN2_STAGES")) : 0;   // diagnostics: shallower weight ring
   if (cap >= 2 && nstage > cap) nstage = cap;
   FQL_REQUIRE(nstage >= 2, "not enough shared memory for the weight pipeline");
   a.nstage = nstage;
-  if (PAIR) a.tiles = (a.tiles + 1) & ~1;     // a pair never straddles two groups: pad the group to an even number of tiles
-  const int smem = fixed + nstage * SLOT;
-  auto kern = mlp_chain2_kernel<MODE, PAIR>;
+  const int smem = fixed + nstage * STAGE_BYTES;
+  auto kern = mlp_chain2_kernel<MODE>;
   static bool attr_set[FQL_MAX_DEVICES] = {};
   const int dev = fql_current_device();
   if (!attr_set[dev]) {
@@ -824,28 +747,9 @@ int launch_chain2_t(const Chain2Args& a0, int nkb_x, int npar, bool ln, const CU
     attr_set[dev] = true;
   }
   const int grid = a.tiles * a.P * a.S * a.E;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(C2_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = PAIR ? 2 : 1;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = PAIR ? 1 : 0;
-  FQL_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, mapX, mapW, mapWL, mapW0, a));
+  kern<<<grid, C2_THREADS, smem, st>>>(mapX, mapW, mapWL, mapW0, a);
   FQL_CHECK_LAUNCH();
   return 0;
-}
-template <int MODE>
-int launch_chain2(const Chain2Args& a, bool pair, int nkb_x, int npar, bool ln, const CUtensorMap& mapX, const CUtensorMap& mapW,
-                  const CUtensorMap& mapWL, const CUtensorMap& mapW0, cudaStream_t st) {
-  if (pair) return launch_chain2_t<MODE, true>(a, nkb_x, npar, ln, mapX, mapW, mapWL, mapW0, st);
-  return launch_chain2_t<MODE, false>(a, nkb_x, npar, ln, mapX, mapW, mapWL, mapW0, st);
 }
 
 }  // namespace
@@ -903,14 +807,13 @@ int tc_mlp_chain2(const TcChainSpec& f, cudaStream_t st) {
   const int64_t x_rows = (int64_t)f.P * a.S * f.Mcap0;
   FQL_TRY(make_map_2d(&mapX, f.X0b, a.K0pad, x_rows, 64, TILE_M));
   static const bool no3d = getenv("FQL_B200_CHAIN2_W3D") && getenv("FQL_B200_CHAIN2_W3D")[0] == '0';
-  const bool pair = chain2_pair(a.tiles);
-  a.w3d = (!pair && !no3d && make_map_w3d(&mapW, f.shadow, (uint64_t)a.S * a.w_rows_s)) ? 1 : 0;
+  a.w3d = (!no3d && make_map_w3d(&mapW, f.shadow, (uint64_t)a.S * a.w_rows_s)) ? 1 : 0;
   if (!a.w3d) FQL_TRY(make_map_2d(&mapW, f.shadow, HID, (uint64_t)a.S * a.w_rows_s, 64, KS));
   FQL_TRY(make_map_2d(&mapWL, f.shadow, 64, (uint64_t)a.S * a.wl_rows_s, 64, KS));
   const int nkb_x = a.K0pad / 64;
-  if (n0.ln) return launch_chain2<C2_FWD_LN>(a, pair, nkb_x, 3, true, mapX, mapW, mapWL, mapWL, st);
-  if (euler) return launch_chain2<C2_EULER>(a, pair, nkb_x, 1, false, mapX, mapW, mapWL, mapWL, st);
-  return launch_chain2<C2_FWD>(a, pair, nkb_x, 1, false, mapX, mapW, mapWL, mapWL, st);
+  if (n0.ln) return launch_chain2<C2_FWD_LN>(a, nkb_x, 3, true, mapX, mapW, mapWL, mapWL, st);
+  if (euler) return launch_chain2<C2_EULER>(a, nkb_x, 1, false, mapX, mapW, mapWL, mapWL, st);
+  return launch_chain2<C2_FWD>(a, nkb_x, 1, false, mapX, mapW, mapWL, mapWL, st);
 }
 
 // The input-gradient chain of one network's backward on M rows per group: dZ_{NL-2} ... dZ_0 as bf16 (operands of the weight
@@ -939,11 +842,9 @@ int tc_mlp_chain2_backward(const TcChain2BwdSpec& f, cudaStream_t st) {
   a.out = f.dX0;
   CUtensorMap mapX, mapW, mapWL, mapW0;
   FQL_TRY(make_map_2d(&mapX, f.dOutb, 64, (uint64_t)a.S * nv.ens * f.M, 64, TILE_M));
-  const bool pair = chain2_pair(a.tiles);
-  const int nc = pair ? 2 : 1;       // a CTA of a pair loads half of the input rows of every W^T stage
-  FQL_TRY(make_map_2d(&mapW, f.shadow, HID, (uint64_t)a.S * a.w_rows_s, KS, NHALF / nc, CU_TENSOR_MAP_SWIZZLE_64B));
-  FQL_TRY(make_map_2d(&mapWL, f.shadow, 64, (uint64_t)a.S * a.wl_rows_s, KS, NHALF / nc, CU_TENSOR_MAP_SWIZZLE_64B));
-  FQL_TRY(make_map_2d(&mapW0, f.shadow, HID, (uint64_t)a.S * a.w_rows_s, KS, a.K0pad / nc, CU_TENSOR_MAP_SWIZZLE_64B));
-  if (nv.ln) return launch_chain2<C2_BWD_LN>(a, pair, 1, 1, true, mapX, mapW, mapWL, mapW0, st);
-  return launch_chain2<C2_BWD>(a, pair, 1, 0, false, mapX, mapW, mapWL, mapW0, st);
+  FQL_TRY(make_map_2d(&mapW, f.shadow, HID, (uint64_t)a.S * a.w_rows_s, KS, NHALF, CU_TENSOR_MAP_SWIZZLE_64B));
+  FQL_TRY(make_map_2d(&mapWL, f.shadow, 64, (uint64_t)a.S * a.wl_rows_s, KS, NHALF, CU_TENSOR_MAP_SWIZZLE_64B));
+  FQL_TRY(make_map_2d(&mapW0, f.shadow, HID, (uint64_t)a.S * a.w_rows_s, KS, a.K0pad, CU_TENSOR_MAP_SWIZZLE_64B));
+  if (nv.ln) return launch_chain2<C2_BWD_LN>(a, 1, 1, true, mapX, mapW, mapWL, mapW0, st);
+  return launch_chain2<C2_BWD>(a, 1, 0, false, mapX, mapW, mapWL, mapW0, st);
 }

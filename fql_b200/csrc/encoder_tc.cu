@@ -26,8 +26,6 @@
 #include "step.cuh"
 #include "tc_prims.cuh"
 
-#include <cudaTypedefs.h>
-
 using namespace tc;
 typedef __nv_bfloat16 bf16;
 
@@ -614,16 +612,6 @@ __global__ void enc_relu_mask_kernel(const float* __restrict__ d, const bf16* __
   if (i < n) out[i] = __float2bfloat16(__bfloat162float(xr[i]) > 0.f ? d[i] : 0.f);
 }
 
-PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
-  static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-  }
-  return fn;
-}
 // prepared weights [rows][64] bf16 as boxes of [32 k][64 n]
 int make_map_w(CUtensorMap* m, const void* base, int rows) {
   auto enc = get_encode();

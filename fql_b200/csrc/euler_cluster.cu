@@ -26,8 +26,6 @@
 #include "step.cuh"
 #include "tc_prims.cuh"
 
-#include <cudaTypedefs.h>
-
 using namespace tc;
 
 namespace {
@@ -111,45 +109,6 @@ __device__ __forceinline__ float gelu_grad_fast(float x) {
 __device__ __forceinline__ uint32_t pack2(float a, float b) {
   __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
   return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire;" ::: "memory");
-}
-// arrive on the mbarrier at the same smem offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint64_t* bar, uint32_t rank) {
-  uint32_t raddr;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(raddr) : "r"(smem_u32(bar)), "r"(rank));
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(raddr) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred P;\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2;\n\tselp.u32 %0, 1, 0, P;\n\t}\n"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-// (loop inside the asm block: see mbar_wait_u in tc_prims.cuh)
-__device__ __forceinline__ void mbar_wait_cluster_u(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t.reg .pred P1, P2;\n\t.reg .u32 c;\n\tmov.u32 c, 0;\n"
-      "WC_LOOP:\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P1, [%0], %1;\n\t@P1 bra WC_DONE;\n\t"
-      "add.u32 c, c, 1;\n\tsetp.lt.u32 P2, c, 0x4000000;\n\t@P2 bra WC_LOOP;\n\ttrap;\n"
-      "WC_DONE:\n\t}\n" ::"r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!mbar_try_wait_cluster(bar, parity)) {
-    if (++spins > (1u << 26)) mbar_timeout(bar, parity);
-  }
 }
 
 // AMAX: compile-time bound of action_dim (the Euler update is unrolled over it; the kernel's code must stay small -- the rarely
@@ -522,32 +481,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) euler_cluster_kernel(const __grid
   cluster_sync_all();  // no CTA may exit while a peer can still arrive on its barriers
   if (a.t_start && blockIdx.x == 0 && threadIdx.x == 0) a.t_start[1] = gtime();
   if (warp == 1) tmem_dealloc(tmem_base, 2 * ACC_SET);
-}
-
-PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
-  static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-  }
-  return fn;
-}
-
-int make_map_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t rows, uint32_t box_inner, uint32_t box_rows,
-                CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B) {
-  auto enc = get_encode();
-  FQL_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is not available from the driver");
-  cuuint64_t dims[2] = {inner, rows};
-  cuuint64_t strides[1] = {inner * 2};
-  cuuint32_t box[2] = {box_inner, box_rows};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  FQL_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (%d) inner=%llu rows=%llu", (int)r, (unsigned long long)inner,
-              (unsigned long long)rows);
-  return 0;
 }
 
 }  // namespace

@@ -27,9 +27,7 @@ __device__ float block_reduce(float v, float* sh) {
 }
 
 // Builds every first-layer input of the step (concats of networks.py:191,229-231) + vel (fql.py:55-56).
-// kF / kO > 0 (tensor-core mode): also write the zero-padded bf16 operands XFb [S][2B][kF] and XOb [S][3B][kO], so that no
-// conversion kernel stands between this kernel and the first GEMMs of the two longest chains
-__global__ void prep_kernel(StepShape sh, FqlBatch b, WsPtrs w, int kF, int kO) {
+__global__ void prep_kernel(StepShape sh, FqlBatch b, WsPtrs w) {
   const int row = blockIdx.x;  // s*B + r
   const int s = row / sh.B, r = row % sh.B;
   const int F = sh.F, A = sh.A, B = sh.B;
@@ -72,23 +70,6 @@ __global__ void prep_kernel(StepShape sh, FqlBatch b, WsPtrs w, int kF, int kO) 
   if (threadIdx.x == 0) {
     xf0[F + A] = t;
     xf1[F + A] = 0.0f;  // Euler step 0: t = 0/flow_steps (fql.py:167)
-  }
-  if (kF > 0) {
-    __syncthreads();  // the fp32 rows above were written by other threads of this block
-    __nv_bfloat16* fb0 = reinterpret_cast<__nv_bfloat16*>(w.XFb) + ((int64_t)s * 2 * B + r) * kF;
-    __nv_bfloat16* fb1 = fb0 + (int64_t)B * kF;
-    for (int c = threadIdx.x; c < kF; c += blockDim.x) {
-      fb0[c] = __float2bfloat16(c < KF ? xf0[c] : 0.f);
-      fb1[c] = __float2bfloat16(c < KF ? xf1[c] : 0.f);
-    }
-    __nv_bfloat16* ob0 = reinterpret_cast<__nv_bfloat16*>(w.XOb) + ((int64_t)s * 3 * B + r) * kO;
-    __nv_bfloat16* ob1 = ob0 + (int64_t)B * kO;
-    __nv_bfloat16* ob2 = ob1 + (int64_t)B * kO;
-    for (int c = threadIdx.x; c < kO; c += blockDim.x) {
-      ob0[c] = __float2bfloat16(c < KO ? xo0[c] : 0.f);
-      ob1[c] = __float2bfloat16(c < KO ? xo1[c] : 0.f);
-      ob2[c] = __float2bfloat16(c < KO ? xo2[c] : 0.f);
-    }
   }
 }
 
@@ -351,8 +332,8 @@ static int loss_ctas(const StepShape& sh) {
   return c < 1 ? 1 : (c > 64 ? 64 : c);
 }
 
-int launch_prep(const StepShape& sh, const FqlBatch& b, const WsPtrs& w, cudaStream_t st, int kF, int kO) {
-  prep_kernel<<<sh.S * sh.B, 64, 0, st>>>(sh, b, w, kF, kO);
+int launch_prep(const StepShape& sh, const FqlBatch& b, const WsPtrs& w, cudaStream_t st) {
+  prep_kernel<<<sh.S * sh.B, 64, 0, st>>>(sh, b, w);
   FQL_CHECK_LAUNCH();
   return 0;
 }

@@ -16,8 +16,6 @@
 #include "step.cuh"
 #include "tc_prims.cuh"
 
-#include <cudaTypedefs.h>
-
 #include <map>
 #include <vector>
 
@@ -418,8 +416,10 @@ __global__ void pad_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __re
   *reinterpret_cast<uint4*>(y + r * K0pad + c0) = make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
 }
 
+}  // namespace
+
 // ---------------------------------------------------------------------------------------------------------------
-// host: tensor maps
+// host: tensor maps (shared by every tensor-core source)
 // ---------------------------------------------------------------------------------------------------------------
 PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
   static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
@@ -432,7 +432,8 @@ PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
   return fn;
 }
 
-int make_map_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t rows, uint32_t box_inner, uint32_t box_rows) {
+int make_map_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t rows, uint32_t box_inner, uint32_t box_rows,
+                CUtensorMapSwizzle swz) {
   auto enc = get_encode();
   FQL_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is not available from the driver");
   cuuint64_t dims[2] = {inner, rows};
@@ -440,13 +441,11 @@ int make_map_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t rows,
   cuuint32_t box[2] = {box_inner, box_rows};
   cuuint32_t es[2] = {1, 1};
   CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                   swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   FQL_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (%d) inner=%llu rows=%llu", (int)r, (unsigned long long)inner,
               (unsigned long long)rows);
   return 0;
 }
-
-}  // namespace
 
 // ---------------------------------------------------------------------------------------------------------------
 // public (library-internal) API

@@ -426,12 +426,8 @@ struct FqlContext {
   int use_graph = 1;
   int use_euler_cluster = 1;
   int use_cluster_fwd = 1;   // FQL_B200_CLUSTER_FWD=0: one-step actor forward layer by layer
-  int fused_prep = 0;        // FQL_B200_FUSED_PREP=1: the prep kernel also writes the bf16 first-layer operands (measured: no gain over
-                             // the two PDL-launched conversion kernels, which run in parallel on their own streams)
   int use_cluster_bwd = 1;   // FQL_B200_CLUSTER_BWD=0: one-step actor dgrad chain layer by layer
   unsigned long long* stamps = nullptr;  // FQL_B200_STAMPS=1: %globaltimer at schedule points (diagnostics, profiles/dbg_timeline.py)
-  int split_adam = 0;        // FQL_B200_SPLIT_ADAM: 0 = one optimizer pass at the end (default: the others measured within noise), 1 = bc-flow's part right behind the Euler chain,
-                             // 2 = bc-flow and critic parts before the one-step actor's gradients are complete
   int adam_done_blk = 0;     // blocks [0, adam_done_blk) were already applied by enqueue_grads_tc in this enqueue
   int euler_hoist = 1;       // FQL_B200_EULER_HOIST=0: pixel configs, Euler integration layer by layer instead of hoisted first layer + cluster kernel
   int enc_streams = 1;       // FQL_B200_ENC_STREAMS=0: pixel configs, the five tensor-core encoder forwards on one stream
@@ -439,7 +435,6 @@ struct FqlContext {
                              // runs behind their bucket reductions, under the one-step actor's bucket exchange
   int dp_bc_late = 0;        // FQL_B200_DP_BC_LATE=1: bc-flow's bucket is exchanged together with the critic's (one launch) instead of
                              // under the Euler chain
-  int use_critic_chain = 0;
   int use_big_bwd = 1;       // FQL_B200_BIG_BWD=0: per-layer backward (tc_gemm + row kernels) also at large batch
   int chain_min_tiles = 48;  // row tiles (x seeds) from which the fused per-tile chain kernels replace the per-layer GEMMs
   cudaEvent_t early_event = nullptr;  // optional: recorded when the bc-flow and critic gradients of fql_step_grads are complete
@@ -534,8 +529,6 @@ extern "C" int fql_context_create(FqlContext** out) {
   if (g && g[0] == '0') c->use_graph = 0;
   const char* ec = getenv("FQL_B200_EULER_CLUSTER");
   if (ec && ec[0] == '0') c->use_euler_cluster = 0;
-  const char* fp = getenv("FQL_B200_FUSED_PREP");
-  if (fp) c->fused_prep = fp[0] == '1';
   const char* cbw = getenv("FQL_B200_CLUSTER_BWD");
   if (cbw && cbw[0] == '0') c->use_cluster_bwd = 0;
   const char* cfw = getenv("FQL_B200_CLUSTER_FWD");
@@ -545,8 +538,6 @@ extern "C" int fql_context_create(FqlContext** out) {
     FQL_CHECK_CUDA(cudaMalloc(&c->stamps, 576 * sizeof(unsigned long long)));  // 64 schedule points + [32 CTAs][16] Euler phases
     FQL_CHECK_CUDA(cudaMemset(c->stamps, 0, 576 * sizeof(unsigned long long)));
   }
-  const char* sa = getenv("FQL_B200_SPLIT_ADAM");
-  if (sa) c->split_adam = atoi(sa);
   const char* ehs = getenv("FQL_B200_EULER_HOIST");
   if (ehs) c->euler_hoist = atoi(ehs);
   const char* ens = getenv("FQL_B200_ENC_STREAMS");
@@ -559,8 +550,6 @@ extern "C" int fql_context_create(FqlContext** out) {
   if (cm) c->chain_min_tiles = atoi(cm);
   const char* bb = getenv("FQL_B200_BIG_BWD");
   if (bb && bb[0] == '0') c->use_big_bwd = 0;
-  const char* cc = getenv("FQL_B200_CRITIC_CHAIN");
-  if (cc && cc[0] == '1') c->use_critic_chain = 1;
   *out = c;
   return 0;
 }
@@ -688,8 +677,7 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
   FQL_TRY(stamp(ctx, 0, S0));   // step start
   FQL_TRY(launch_zero_bc(raw, (int64_t)S * FQL_NUM_RAW, c.do_apply ? c.st->count : nullptr, hp, w.gstats + S * 4, S0, w.cpost_ticket, 3 * S));
   FQL_TRY(encode_observations(c, L, w, S0, ctx));
-  const bool fused_prep = ctx->fused_prep;
-  FQL_TRY(launch_prep(sh, b, w, S0, fused_prep ? kF : 0, fused_prep ? kO : 0));  // also writes the bf16 first-layer operands XFb / XOb
+  FQL_TRY(launch_prep(sh, b, w, S0));
   FQL_TRY(stamp(ctx, 1, S0));   // prep done
   FQL_CHECK_CUDA(cudaEventRecord(ev_prep, S0));
   FQL_CHECK_CUDA(cudaStreamWaitEvent(S1, ev_prep, 0));
@@ -709,7 +697,7 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
   };
 
   // ---- S1: Euler (agents/fql.py:155-171) on rows [B, 2B) of the bc-flow buffers
-  if (!fused_prep) FQL_TRY(tc_pad_bf16(w.XF, w.XFb, (int64_t)S * 2 * B, sh.F + sh.A + 1, kF, S1));
+  FQL_TRY(tc_pad_bf16(w.XF, w.XFb, (int64_t)S * 2 * B, sh.F + sh.A + 1, kF, S1));
   FQL_CHECK_CUDA(cudaEventRecord(ev_pad, S1));
   const int row_tiles = S * ((B + 127) / 128);
   const bool many_tiles = row_tiles >= ctx->chain_min_tiles && !wide;  // enough 128-row tiles to fill the GPU: fused per-tile chain kernels
@@ -816,9 +804,9 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
   (void)ev_f0;
 
   // ---- S0: one-step actor on {(s',z_next), (s,z), (s,z')}, grouped critic pass
-  if (!fused_prep) FQL_TRY(tc_pad_bf16(w.XO, w.XOb, (int64_t)S * 3 * B, sh.F + sh.A, kO, S0));
+  FQL_TRY(tc_pad_bf16(w.XO, w.XOb, (int64_t)S * 3 * B, sh.F + sh.A, kO, S0));
   TcActor fo = actor(FQL_NET_ACTOR_ONESTEP_FLOW, w.XOb, kO, 3 * B, 0, 3 * B, w.O_Hb, w.O_Zb, true);
-  bool split_metric = false, early_adam_s1 = false;
+  bool split_metric = false;
   if (many_tiles) {
     FQL_TRY(chain(FQL_NET_ACTOR_ONESTEP_FLOW, w.XOb, 3 * B, 0, 3 * B, w.O_Hb, w.O_Zb, w.O_out, 1, S0));
   } else {
@@ -854,7 +842,7 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
   cr.d = d; cr.L = &L; cr.params = P; cr.shadow = shadow; cr.M = B; cr.K0pad = kO; cr.x_ss = (long long)B * kO; cr.buf = &w.pC; cr.Hb = w.C_Hb;
   cr.cs_scratch = w.cs_scratch[2];
   bool split_cpost = false;
-  if ((ctx->use_critic_chain && !wide) || many_tiles) {   // enough row tiles to fill the GPU: the three critic problems x 2 heads as ONE fused launch
+  if (many_tiles) {   // enough row tiles to fill the GPU: the three critic problems x 2 heads as ONE fused launch
     TcChainSpec t;
     memset(&t, 0, sizeof(t));
     t.d = d; t.L = &L; t.P = 3; t.net[0] = FQL_NET_TARGET_CRITIC; t.net[1] = FQL_NET_CRITIC; t.net[2] = FQL_NET_CRITIC;
@@ -930,7 +918,7 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
     if (big_bwd) FQL_TRY(tc_critic_backward_big(q, w.C_XHb, w.C_DGb, S0));
     else FQL_TRY(tc_critic_backward(q, S0, nullptr, nullptr, &ctx->ev[44]));
     FQL_TRY(stamp(ctx, 6, S0));   // critic input-gradient chain done
-    if (dp_bucketed && c.do_apply && ctx->dp_early_adam && ctx->split_adam == 0 && d->reserved[0] == 0) {
+    if (dp_bucketed && c.do_apply && ctx->dp_early_adam) {
       // data parallel: bc-flow's and the critic's part of the optimizer pass (+ Polyak) right behind their bucket exchanges on the
       // communication stream, under the one-step actor's backward and bucket exchange.  Last readers of their weights: the Euler
       // chain (bc-flow) and the critic input-gradient chain that S0 has just enqueued; the critic's own backward precedes ev[36].
@@ -943,31 +931,6 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
       FQL_TRY(stamp(ctx, 9, ctx->sc));  // early optimizer pass done
       FQL_CHECK_CUDA(cudaEventRecord(ctx->ev[59], ctx->sc));
       ctx->adam_done_blk = blk1;
-    }
-    if (c.do_apply && ctx->split_adam == 1 && d->reserved[0] == 0) {
-      // bc-flow is finished with once the Euler chain (the last reader of its weights) has ended and its gradients are complete:
-      // its quarter of the optimizer pass runs behind the Euler kernel, beside the one-step actor's dgrad chain
-      const int blk0 = (int)(L.net[FQL_NET_CRITIC].begin / FQL_LEAF_PAD);
-      FQL_CHECK_CUDA(cudaStreamWaitEvent(S1, ctx->ev[16], 0));
-      FQL_TRY(launch_adam_polyak_stats(L, hp, S, c.st->params, c.st->mu, c.st->nu, c.st->grads, w.gstats + S * 4, w.partials, c.st->shadow,
-                                       tc_shadow_seed_elems(d, L), S1, 0, blk0));
-      FQL_TRY(stamp(ctx, 9, S1)); // early optimizer pass done
-      FQL_CHECK_CUDA(cudaEventRecord(ctx->ev[58], S1));
-      early_adam_s1 = true;
-      ctx->adam_done_blk = blk0;
-    }
-    if (c.do_apply && ctx->split_adam == 2 && d->reserved[0] == 0) {
-      // (measured slower than mode 1: the critic's half of the pass then competes with the one-step actor's parameter gradients)
-      FQL_CHECK_CUDA(cudaEventRecord(ctx->ev[52], S0));
-      FQL_CHECK_CUDA(cudaStreamWaitEvent(S2, ctx->ev[52], 0));
-      const int blk0 = (int)(L.net[FQL_NET_CRITIC].begin / FQL_LEAF_PAD), blk1 = (int)(L.net[FQL_NET_ACTOR_ONESTEP_FLOW].begin / FQL_LEAF_PAD);
-      FQL_TRY(launch_adam_polyak_stats(L, hp, S, c.st->params, c.st->mu, c.st->nu, c.st->grads, w.gstats + S * 4, w.partials, c.st->shadow,
-                                       tc_shadow_seed_elems(d, L), S2, blk0, blk1));   // critic (+ Polyak into the target)
-      FQL_CHECK_CUDA(cudaStreamWaitEvent(S2, ev_euler, 0));
-      FQL_TRY(launch_adam_polyak_stats(L, hp, S, c.st->params, c.st->mu, c.st->nu, c.st->grads, w.gstats + S * 4, w.partials, c.st->shadow,
-                                       tc_shadow_seed_elems(d, L), S2, 0, blk0));      // bc-flow: the Euler chain was its last reader
-      ctx->adam_done_blk = blk1;
-      FQL_TRY(stamp(ctx, 9, S2)); // early optimizer pass done
     }
   }
   if (bc_enc_forked) FQL_CHECK_CUDA(cudaStreamWaitEvent(S2, ctx->ev[37], 0));
@@ -1018,7 +981,6 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
     FQL_TRY(stamp(ctx, 10, S0));  // one-step actor gradients complete
   }
   FQL_CHECK_CUDA(cudaStreamWaitEvent(S0, ev_s2, 0));
-  if (early_adam_s1) FQL_CHECK_CUDA(cudaStreamWaitEvent(S0, ctx->ev[58], 0));
   if (dp_grads && !dp_bucketed) {
     const int64_t t0 = L.net[FQL_NET_TARGET_CRITIC].begin;
     FQL_TRY(dp_reduce_bucket(ctx->dp, 3, 0, t0, raw, S0));

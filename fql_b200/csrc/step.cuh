@@ -2,6 +2,8 @@
 #pragma once
 #include "common.cuh"
 
+#include <cudaTypedefs.h>
+
 enum {  // raw accumulators per seed (all-reduced across data-parallel ranks: [0..8] SUM, [9..10] MAX)
   RAW_CRITIC_SQ = 0, RAW_Q_SUM = 1, RAW_BC_SQ = 2, RAW_DISTILL_SQ = 3, RAW_QPI_SUM = 4, RAW_QPI_ABS = 5, RAW_MSE = 6,
   RAW_Q_MAX = 9, RAW_Q_NEGMIN = 10,
@@ -69,7 +71,7 @@ struct WsPtrs {
 StepShape make_shape(const FqlDims* d);
 size_t carve_workspace(const FqlDims* d, const Layout& L, void* base, WsPtrs* w);  // returns bytes needed
 
-int launch_prep(const StepShape& sh, const FqlBatch& b, const WsPtrs& w, cudaStream_t st, int kF = 0, int kO = 0);
+int launch_prep(const StepShape& sh, const FqlBatch& b, const WsPtrs& w, cudaStream_t st);
 int launch_post_onestep(const StepShape& sh, const FqlBatch& b, const WsPtrs& w, float* raw, cudaStream_t st, int parts = 3);
 struct DpLamArgs;
 int launch_critic_post(const StepShape& sh, const FqlHparams& hp, const FqlBatch& b, const WsPtrs& w, float* raw, cudaStream_t st, int parts = 3,
@@ -195,6 +197,11 @@ int tc_pad_bf16(const float* x, void* y, int64_t rows, int K0, int K0pad, cudaSt
 int tc_mlp_chain(const TcChainSpec& f, cudaStream_t st);
 int tc_mlp_chain2_supported(const FqlDims* d);
 int tc_mlp_chain2(const TcChainSpec& f, cudaStream_t st);
+// TMA tensor maps: the driver's cuTensorMapEncodeTiled (NULL when the driver does not provide it), and a bf16 [rows][inner] row-major
+// tensor read in boxes of [box_rows][box_inner]
+PFN_cuTensorMapEncodeTiled_v12000 get_encode();
+int make_map_2d(CUtensorMap* m, const void* base, uint64_t inner, uint64_t rows, uint32_t box_inner, uint32_t box_rows,
+                CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B);
 
 // tc_gemm.cu -- generic tcgen05 GEMM (one Dense layer: forward / dgrad / wgrad)
 enum { TC_MODE_STORE_F32 = 0, TC_MODE_FWD_HIDDEN = 1, TC_MODE_DGRAD_GELU = 2, TC_MODE_EULER = 3, TC_MODE_WGRAD_LN = 4 };

@@ -14,7 +14,6 @@
 #include "step.cuh"
 #include "tc_prims.cuh"
 
-#include <cudaTypedefs.h>
 #include <stdlib.h>
 
 using namespace tc;
@@ -354,17 +353,6 @@ __global__ void __launch_bounds__(NTHREADS, 1) tc_gemm_kernel(const __grid_const
   __syncthreads();
   if (warp == 1) tmem_dealloc(tmem_base, 64 * NACC);
   if (dbg && threadIdx.x == 32) dbg[6] = gtime();
-}
-
-PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
-  static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-  }
-  return fn;
 }
 
 int make_map_4d(CUtensorMap* m, const TcOperand& o, uint32_t box_rows) {

@@ -61,6 +61,26 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
+// ---- thread-block cluster ----------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ void cluster_sync_all() {
+  asm volatile("barrier.cluster.arrive.release;" ::: "memory");
+  asm volatile("barrier.cluster.wait.acquire;" ::: "memory");
+}
+// mbar_wait_u for a barrier that takes arrivals from other CTAs of the cluster (acquire at cluster scope)
+__device__ __forceinline__ void mbar_wait_cluster_u(uint64_t* bar, uint32_t parity) {
+  asm volatile(
+      "{\n\t.reg .pred P1, P2;\n\t.reg .u32 c;\n\tmov.u32 c, 0;\n"
+      "WC_LOOP:\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P1, [%0], %1;\n\t@P1 bra WC_DONE;\n\t"
+      "add.u32 c, c, 1;\n\tsetp.lt.u32 P2, c, 0x4000000;\n\t@P2 bra WC_LOOP;\n\ttrap;\n"
+      "WC_DONE:\n\t}\n" ::"r"(smem_u32(bar)), "r"(parity)
+      : "memory");
+}
+
 // ---- TMA --------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* m) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
@@ -127,79 +147,6 @@ __device__ __forceinline__ void umma_bf16_x2(uint32_t d_tmem, uint64_t a_desc, u
       ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate_first), "l"(a_step), "l"(b_step)
       : "memory");
 }
-// ---- CTA pair (cta_group::2): one MMA covers M = 256 rows, 128 from each CTA of a 2-CTA cluster; issued by the leader (rank 0) only.
-// A: each CTA's own [128 rows][K] tile at the SAME smem offset; B: each CTA holds half of the N columns (rank r: [r N/2, (r+1) N/2)).
-__device__ __forceinline__ void umma2_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma2_bf16_x2(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint64_t a_step, uint64_t b_step,
-                                              uint32_t idesc, uint32_t accumulate_first) {
-  asm volatile(
-      "{\n\t.reg .pred p, q;\n\t.reg .b64 a1, b1;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "setp.eq.b32 q, 0, 0;\n\t"
-      "add.u64 a1, %1, %5;\n\tadd.u64 b1, %2, %6;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], a1, b1, %3, q;\n\t}\n"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate_first), "l"(a_step), "l"(b_step)
-      : "memory");
-}
-// arrive on the mbarrier at this smem offset in BOTH CTAs of the pair when all previously issued MMAs have completed
-__device__ __forceinline__ void umma2_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"((uint16_t)3)
-               : "memory");
-}
-__device__ __forceinline__ void tmem_alloc2(uint32_t* dst_smem, uint32_t cols) {  // one full warp in EACH CTA of the pair
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t cols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-// TMA load whose completion bytes go to the mbarrier at the same offset in the LEADER CTA of the pair (executed by either CTA)
-__device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & 0xFEFFFFFFu), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank_() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_() {
-  asm volatile("barrier.cluster.arrive.release;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire;" ::: "memory");
-}
-// arrive (release at cluster scope) on the mbarrier at the same smem offset in CTA `rank` of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint64_t* bar, uint32_t rank) {
-  uint32_t raddr;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(raddr) : "r"(smem_u32(bar)), "r"(rank));
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(raddr) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait_cl(uint64_t* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred P;\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2;\n\tselp.u32 %0, 1, 0, P;\n\t}\n"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait_cl(uint64_t* bar, uint32_t parity) {   // a barrier with arrivals from the peer CTA
-  uint32_t spins = 0;
-  while (!mbar_try_wait_cl(bar, parity)) {
-    if (++spins > (1u << 26)) mbar_timeout(bar, parity);
-  }
-}
-__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
-
 // arrive on an mbarrier when all previously issued tcgen05.mma of this thread have completed (implies fence::before)
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");

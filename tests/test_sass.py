@@ -61,9 +61,6 @@ def test_contractions_are_tcgen05_tmem_tma(sass_counts):
 
 
 def test_single_thread_roles_are_warp_uniform(sass_counts):
-    # cta_group::2 (PAIR = true) instantiations of the chain kernel are opt-in diagnostics and take their rank from %cluster_ctarank
     for fam in ('euler_cluster_kernel', 'mlp_chain2_kernel', 'tc_gemm_kernel', 'conv_tc_kernel', 'mlp_chain_tc_kernel'):
         for name, c in _family(sass_counts, fam).items():
-            if fam == 'mlp_chain2_kernel' and 'Lb1E' in name:
-                continue
             assert c['bcast'] <= max(12, c['mma'] // 4), (name, c)

@@ -124,16 +124,12 @@ def test_tc_update_two_seeds_cluster_kernels():
 
 
 SWITCHES = [
-    dict(FQL_B200_CRITIC_CHAIN='1'),                                  # critic forward: fused chain kernel, LayerNorm in the TMEM epilogue
     dict(FQL_B200_CLUSTER_FWD='0', FQL_B200_CLUSTER_BWD='0'),         # one-step actor layer by layer
     dict(FQL_B200_EULER_CLUSTER='0'),                                 # Euler integration layer by layer (tc_gemm Euler epilogue)
     dict(FQL_B200_CHAIN_MIN_TILES='1'),                               # large-batch routing: fused per-tile chain kernels everywhere
     dict(FQL_B200_CHAIN_MIN_TILES='1', FQL_B200_BIG_BWD='0'),         # ... with the per-layer backward (tc_gemm + LayerNorm row kernels)
     dict(FQL_B200_CHAIN_MIN_TILES='1', FQL_B200_CHAIN2='0'),          # ... with the non-overlapped chain kernel (mlp_tc.cu)
     dict(FQL_B200_CHAIN_MIN_TILES='1', FQL_B200_CHAIN2_W3D='0'),      # ... with four 2-D weight boxes per stage instead of one 3-D box
-    dict(FQL_B200_SPLIT_ADAM='1'),
-    dict(FQL_B200_SPLIT_ADAM='2'),
-    dict(FQL_B200_FUSED_PREP='1'),
     dict(FQL_B200_GRAPH='0'),                                         # every step enqueued eagerly
 ]
 

@@ -82,17 +82,3 @@ def test_tc_64_seeds_puzzle():
         for k in ('critic/critic_loss', 'actor/bc_flow_loss', 'actor/distill_loss', 'actor/q_loss'):
             info_close(k, info[k][s], refs[which[s]][1], 5e-2)
 
-
-def test_tc_large_batch_update_cta_pairs():
-    """The same large-batch cases with the chain kernels as cta_group::2 CTA pairs (FQL_B200_CHAIN2_PAIR=1, opt-in: measured slower than
-    one CTA per tile, kept as the base of the two-issuer design).  The switch is read once per process: run in a child process."""
-    import os
-    import subprocess
-    import sys
-    if os.environ.get('FQL_B200_CHAIN2_PAIR') == '1':
-        pytest.skip('already inside the CTA-pair run')
-    env = dict(os.environ, FQL_B200_CHAIN2_PAIR='1')
-    r = subprocess.run([sys.executable, '-m', 'pytest', os.path.abspath(__file__), '-m', 'gpu', '-q', '-x', '-k', 'B8192 or B1000 or 64_seeds'],
-                       env=env, capture_output=True, text=True, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))), timeout=900)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-    assert '3 passed' in r.stdout, r.stdout[-1000:]
