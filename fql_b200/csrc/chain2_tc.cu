@@ -1,8 +1,8 @@
 // chain2_tc.cu -- the throughput variant of the fused MLP chain (hidden = 512): one CTA runs a whole MLP forward -- for
 // compute_flow_actions (agents/fql.py:155-171) the whole Euler loop -- or the whole input-gradient chain of its backward on a
 // 128-row tile, with the epilogue of one layer overlapped with the tensor-core work of the same and the next layer.  Used
-// where seeds x 128-row tiles fill the GPU (batch >= 1024-ish, vectorised seeds: BASELINE configs 3 and 4); mlp_tc.cu keeps
-// the narrower widths and euler_cluster.cu the batch-256 latency path.
+// where seeds x 128-row tiles fill the GPU (batch >= 1024-ish, vectorised seeds: BASELINE configs 3 and 4); euler_cluster.cu
+// keeps the batch-256 latency path, and narrower widths run layer by layer through tc_gemm (tc_path.cu).
 //
 // The 128 x 512 fp32 accumulator of a layer is all of an SM's TMEM, so it cannot be double-buffered across layers.  Instead a
 // layer is issued as two N-halves (TMEM columns [0,256) and [256,512)) and the K loop of the second half runs while the
@@ -753,14 +753,6 @@ int launch_chain2(const Chain2Args& a0, int nkb_x, int npar, bool ln, const CUte
 }
 
 }  // namespace
-
-int tc_mlp_chain2_supported(const FqlDims* d) {
-  static const int on = []() {
-    const char* e = getenv("FQL_B200_CHAIN2");
-    return !(e && e[0] == '0');
-  }();
-  return on && d->hidden == HID;
-}
 
 int tc_mlp_chain2(const TcChainSpec& f, cudaStream_t st) {
   const FqlDims* d = f.d;

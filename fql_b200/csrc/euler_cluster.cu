@@ -1,7 +1,7 @@
 // euler_cluster.cu -- compute_flow_actions (agents/fql.py:155-171) as ONE persistent thread-block-cluster kernel.
 //
 // The Euler integration is the longest dependent chain of an update: flow_steps x 5 Dense layers on the same rows.  At
-// batch 256 that is only two 128-row tiles, so the per-row-tile fused kernel (mlp_tc.cu) leaves 146 SMs idle and a
+// batch 256 that is only two 128-row tiles, so the per-row-tile fused kernel (chain2_tc.cu) leaves 146 SMs idle and a
 // kernel-per-layer schedule pays a launch + pipeline-fill per layer.  Here a cluster of NC (16, or 8 when the GPU cannot
 // hold enough clusters of 16) CTAs owns one 128-row tile:
 //

@@ -140,12 +140,12 @@ struct Carver {
   }
 };
 
-void carve_pass(Carver& c, PassBuf* pb, int G, int Mcap, int H, int NH, int out_dim, bool ln, bool need_z) {
+void carve_pass(Carver& c, PassBuf* pb, int G, int Mcap, int H, int NH, int out_dim, bool ln, bool need_z, bool need_h = true) {
   pb->G = G;
   pb->Mcap = Mcap;
   for (int l = 0; l < NH; l++) {
     pb->Z[l] = (need_z || ln) ? c.take((int64_t)G * Mcap * H) : nullptr;
-    pb->Hh[l] = c.take((int64_t)G * Mcap * H);
+    pb->Hh[l] = need_h ? c.take((int64_t)G * Mcap * H) : nullptr;
     pb->mu[l] = ln ? c.take((int64_t)G * Mcap) : nullptr;
     pb->rstd[l] = ln ? c.take((int64_t)G * Mcap) : nullptr;
   }
@@ -162,9 +162,11 @@ size_t carve_workspace(const FqlDims* d, const Layout& L, void* base, WsPtrs* w)
   w->XF = c.take(S * 2 * B * (F + A + 1));
   w->XC = c.take(3 * S * B * (F + A));
   w->vel = c.take(S * B * A);
-  carve_pass(c, &w->pO, (int)S, (int)(3 * B), (int)H, NH, (int)A, d->actor_layer_norm, true);
-  carve_pass(c, &w->pF, (int)S, (int)(2 * B), (int)H, NH, (int)A, d->actor_layer_norm, true);
-  carve_pass(c, &w->pC, (int)(3 * S * 2), (int)B, (int)H, NH, 1, d->critic_layer_norm, true);
+  // fp32 post-activations: only the SIMT MLPs read them; the tensor-core step keeps bf16 copies (O_Hb, F_Hb, C_Hb below)
+  const bool simt = d->precision != FQL_PRECISION_BF16_TC;
+  carve_pass(c, &w->pO, (int)S, (int)(3 * B), (int)H, NH, (int)A, d->actor_layer_norm, true, simt);
+  carve_pass(c, &w->pF, (int)S, (int)(2 * B), (int)H, NH, (int)A, d->actor_layer_norm, true, simt);
+  carve_pass(c, &w->pC, (int)(3 * S * 2), (int)B, (int)H, NH, 1, d->critic_layer_norm, true, simt);
   w->O_out = w->pO.out;
   w->F_out = w->pF.out;
   w->C_out = w->pC.out;
@@ -436,7 +438,7 @@ struct FqlContext {
   int dp_bc_late = 0;        // FQL_B200_DP_BC_LATE=1: bc-flow's bucket is exchanged together with the critic's (one launch) instead of
                              // under the Euler chain
   int use_big_bwd = 1;       // FQL_B200_BIG_BWD=0: per-layer backward (tc_gemm + row kernels) also at large batch
-  int chain_min_tiles = 48;  // row tiles (x seeds) from which the fused per-tile chain kernels replace the per-layer GEMMs
+  int chain_min_tiles = 48;  // row tiles (x seeds) from which the fused per-tile chain kernels (hidden 512) replace the per-layer GEMMs
   cudaEvent_t early_event = nullptr;  // optional: recorded when the bc-flow and critic gradients of fql_step_grads are complete
   long long launches = 0;  // kernels enqueued through this context
 };
@@ -652,8 +654,8 @@ int encoder_grads(const StepCall& c, const Layout& L, const WsPtrs& w, int net, 
 // FQL_PRECISION_BF16_TC schedule of the loss/gradient half of the step: every contraction on tcgen05.
 //   S1: Euler integration, layer by layer (each layer = 16 CTAs of tc_gemm at B=256)              <- longest chain
 //   S2: bc-flow forward on the BC rows, BC loss, bc-flow backward; then the critic backward
-//   S0: one-step actor forward, grouped critic forward (fused chain kernel, LayerNorm in the epilogue), TD/Q post,
-//       critic input gradient, [join Euler] distillation, one-step actor backward
+//   S0: one-step actor forward, grouped critic forward (tc_gemm + LayerNorm row kernel per layer; at large batch one fused
+//       chain launch, LayerNorm in the epilogue), TD/Q post, critic input gradient, [join Euler] distillation, one-step actor backward
 // ---------------------------------------------------------------------------------------------------------
 int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs& w, const StepShape& sh, const FqlHparams& hp,
                      float* raw, cudaStream_t S0) {
@@ -700,9 +702,11 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
   FQL_TRY(tc_pad_bf16(w.XF, w.XFb, (int64_t)S * 2 * B, sh.F + sh.A + 1, kF, S1));
   FQL_CHECK_CUDA(cudaEventRecord(ev_pad, S1));
   const int row_tiles = S * ((B + 127) / 128);
-  const bool many_tiles = row_tiles >= ctx->chain_min_tiles && !wide;  // enough 128-row tiles to fill the GPU: fused per-tile chain kernels
+  // enough 128-row tiles to fill the GPU: fused per-tile chain kernels (chain2_tc.cu, hidden 512 only; narrower MLPs run layer by
+  // layer at every batch size)
+  const bool many_tiles = H == 512 && row_tiles >= ctx->chain_min_tiles && !wide;
   // ... and the whole backward as chain launches on bf16 gelu' / xhat saves (chain2_tc.cu, tc_path.cu "large-batch backward")
-  const bool big_bwd = many_tiles && ctx->use_big_bwd && tc_mlp_chain2_supported(d) && d->critic_layer_norm && d->reserved[0] == 0;
+  const bool big_bwd = many_tiles && ctx->use_big_bwd && d->critic_layer_norm && d->reserved[0] == 0;
   auto chain = [&](int net, const void* X0b, int rows_cap, int r0_in, int M, void* const* Hb, void* const* Zb, float* out, int n_steps,
                    cudaStream_t st) {
     TcChainSpec t;
@@ -711,7 +715,7 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
     t.r0 = r0_in; t.Hb = Hb; t.Zb = Zb; t.Mcap_override = rows_cap; t.out_override = out; t.n_steps = n_steps;
     if (big_bwd && Zb) { t.DGb = Zb; t.Zb = nullptr; }   // the pre-activation buffers hold gelu'(z) on this path
     if (n_steps > 1) { t.a0 = b.z; t.target = w.target; }
-    return tc_mlp_chain(t, st);
+    return tc_mlp_chain2(t, st);
   };
   if (many_tiles) {
     FQL_TRY(chain(FQL_NET_ACTOR_BC_FLOW, w.XFb, 2 * B, B, B, nullptr, nullptr, nullptr, sh.flow_steps, S1));
@@ -848,7 +852,7 @@ int enqueue_grads_tc(FqlContext* ctx, const StepCall& c, const Layout& L, WsPtrs
     t.d = d; t.L = &L; t.P = 3; t.net[0] = FQL_NET_TARGET_CRITIC; t.net[1] = FQL_NET_CRITIC; t.net[2] = FQL_NET_CRITIC;
     t.params = P; t.shadow = shadow; t.M = B; t.X0b = w.XCb; t.Mcap0 = B; t.buf = &w.pC; t.save = 1; t.n_steps = 1; t.Hb = w.C_Hb;
     if (big_bwd) { t.DGb = w.C_DGb; t.XHb = w.C_XHb; t.save_mask = 6; }   // problems 1 (critic loss) and 2 (actor Q loss) have a backward
-    FQL_TRY(tc_mlp_chain(t, S0));
+    FQL_TRY(tc_mlp_chain2(t, S0));
   } else {
     // three independent chains {target critic(s',a'), critic(s,a), critic(s,clip a_pi)}: S0 + two forked streams
     FQL_CHECK_CUDA(cudaEventRecord(ctx->ev[40], S0));
@@ -1288,31 +1292,53 @@ extern "C" int fql_total_loss(FqlContext* ctx, const FqlDims* d, const FqlHparam
 // standalone forward entry points
 // ---------------------------------------------------------------------------------------------------------
 namespace {
-size_t carve_forward(const FqlDims* d, int rows, int ens, int in_dim, int out_dim, bool ln, void* base, float** X, PassBuf* pb,
-                     void** Xb = nullptr, void** Hx = nullptr, float** feat = nullptr, EncBuf* eb = nullptr) {
+struct FwdWs {          // workspace of the stand-alone forward entry points
+  float* X;             // fp32 first-layer input [S][rows][in_dim]
+  void* Xb;             // bf16 copy, zero padded to K0pad <= 128 columns (tensor cores)
+  void* Hx;             // exchange scratch of the cluster Euler kernel (tensor cores, hidden = 512)
+  void* Hb[FQL_MAXL];   // bf16 hidden activations [S][rows][H] per hidden layer (tensor cores, hidden < 512: layer by layer)
+  float* act;           // fp32 Euler state [S][rows][A] of the same
+  float* feat;          // pixel observations: encoder output and pass buffers
+  EncBuf eb;
+  PassBuf pb;           // fp32 activations / output of the SIMT path
+};
+
+size_t carve_forward(const FqlDims* d, int rows, int ens, int in_dim, int out_dim, bool ln, void* base, FwdWs* f) {
   Carver c{reinterpret_cast<char*>(base)};
-  *X = c.take((int64_t)d->num_seeds * rows * in_dim);
-  void* xb = c.take((int64_t)d->num_seeds * rows * 128 / 2 + 4);
-  if (Xb) *Xb = xb;
-  void* hx = (d->precision == FQL_PRECISION_BF16_TC && d->hidden == 512) ? c.take((int64_t)(tc_euler_scratch_elems(d, rows) / 2 + 4)) : nullptr;
-  if (Hx) *Hx = hx;
-  if (d->reserved[0] > 0) {  // pixel observations: encoder pass buffers + its output
-    float* ft = c.take((int64_t)rows * d->obs_dim);
-    if (feat) *feat = ft;
-    c.off = (c.off + 255) & ~(size_t)255;
-    EncBuf tmp;
-    c.off += enc_carve(d, rows, base ? c.base + c.off : nullptr, eb ? eb : &tmp, false);
+  memset(f, 0, sizeof(*f));
+  f->X = c.take((int64_t)d->num_seeds * rows * in_dim);
+  f->Xb = c.take((int64_t)d->num_seeds * rows * 128 / 2 + 4);
+  const bool tc = d->precision == FQL_PRECISION_BF16_TC;
+  if (tc && d->hidden == 512) f->Hx = c.take((int64_t)(tc_euler_scratch_elems(d, rows) / 2 + 4));
+  if (tc && d->hidden < 512) {
+    for (int l = 0; l < d->num_hidden; l++) f->Hb[l] = c.take((int64_t)d->num_seeds * rows * d->hidden / 2);
+    f->act = c.take((int64_t)d->num_seeds * rows * d->action_dim);
   }
-  carve_pass(c, pb, d->num_seeds * ens, rows, d->hidden, d->num_hidden, out_dim, ln, false);
+  if (d->reserved[0] > 0) {  // pixel observations: encoder pass buffers + its output
+    f->feat = c.take((int64_t)rows * d->obs_dim);
+    c.off = (c.off + 255) & ~(size_t)255;
+    c.off += enc_carve(d, rows, base ? c.base + c.off : nullptr, &f->eb, false);
+  }
+  carve_pass(c, &f->pb, d->num_seeds * ens, rows, d->hidden, d->num_hidden, out_dim, ln, false);
   return c.off + 256;
+}
+
+// the one-step / bc-flow actor layer by layer on the tensor cores (hidden < 512), first-layer operand f.Xb
+TcActor fwd_actor(const FqlDims* d, const Layout& L, int net, const float* params, const void* shadow, int rows, const FwdWs& f) {
+  TcActor t;
+  memset(&t, 0, sizeof(t));
+  t.d = d; t.L = &L; t.net = net; t.params = params; t.shadow = shadow; t.M = rows;
+  t.X0b = f.Xb; t.K0pad = (int)round_up64(L.net[net].in_dim, 64); t.x_ss = (long long)rows * t.K0pad;
+  for (int l = 0; l < d->num_hidden; l++) t.Hb[l] = f.Hb[l];
+  t.h_ss = (long long)rows * d->hidden;
+  return t;
 }
 }  // namespace
 
 extern "C" size_t fql_forward_workspace_bytes(const FqlDims* d, int32_t rows) {
   if (fql_validate_dims(d)) return 0;
-  float* X;
-  PassBuf pb;
-  return carve_forward(d, rows, 2, d->obs_dim + d->action_dim + 1, d->action_dim > 1 ? d->action_dim : 1, true, nullptr, &X, &pb);
+  FwdWs f;
+  return carve_forward(d, rows, 2, d->obs_dim + d->action_dim + 1, d->action_dim > 1 ? d->action_dim : 1, true, nullptr, &f);
 }
 
 static int forward_net(const FqlDims* d, const Layout& L, int net, const float* params, const float* X, PassBuf* pb, int rows,
@@ -1331,14 +1357,13 @@ extern "C" int fql_mlp_forward(FqlContext*, const FqlDims* d, int32_t net, const
   FQL_REQUIRE(net >= 0 && net < FQL_NUM_NETS && rows >= 1, "bad net/rows");
   FQL_REQUIRE(d->precision == FQL_PRECISION_FP32, "fql_mlp_forward: FP32 only");
   const NetView& nv = L.net[net];
-  float* X;
-  PassBuf pb;
-  const size_t need = carve_forward(d, rows, nv.ens, nv.in_dim, nv.out_dim, nv.ln, nullptr, &X, &pb);
+  FwdWs f;
+  const size_t need = carve_forward(d, rows, nv.ens, nv.in_dim, nv.out_dim, nv.ln, nullptr, &f);
   FQL_REQUIRE(workspace && ws_bytes >= need, "workspace too small: have %zu need %zu", ws_bytes, need);
-  carve_forward(d, rows, nv.ens, nv.in_dim, nv.out_dim, nv.ln, workspace, &X, &pb);
+  carve_forward(d, rows, nv.ens, nv.in_dim, nv.out_dim, nv.ln, workspace, &f);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  FQL_TRY(forward_net(d, L, net, params, x, &pb, rows, st));
-  FQL_CHECK_CUDA(cudaMemcpyAsync(y, pb.out, sizeof(float) * (size_t)d->num_seeds * nv.ens * rows * nv.out_dim,
+  FQL_TRY(forward_net(d, L, net, params, x, &f.pb, rows, st));
+  FQL_CHECK_CUDA(cudaMemcpyAsync(y, f.pb.out, sizeof(float) * (size_t)d->num_seeds * nv.ens * rows * nv.out_dim,
                                  cudaMemcpyDeviceToDevice, st));
   return 0;
 }
@@ -1350,33 +1375,33 @@ extern "C" int fql_sample_actions(FqlContext*, const FqlDims* d, const float* pa
   FQL_TRY(fql_build_layout(d, &L));
   FQL_REQUIRE(rows >= 1, "rows=%d", rows);
   const NetView& nv = L.net[FQL_NET_ACTOR_ONESTEP_FLOW];
-  float* X;
-  void* Xb;
-  PassBuf pb;
-  const size_t need = carve_forward(d, rows, 1, nv.in_dim, nv.out_dim, nv.ln, nullptr, &X, &pb);
+  FwdWs f;
+  const size_t need = carve_forward(d, rows, 1, nv.in_dim, nv.out_dim, nv.ln, nullptr, &f);
   FQL_REQUIRE(workspace && ws_bytes >= need, "workspace too small: have %zu need %zu", ws_bytes, need);
-  float* feat = nullptr;
-  EncBuf eb;
-  carve_forward(d, rows, 1, nv.in_dim, nv.out_dim, nv.ln, workspace, &X, &pb, &Xb, nullptr, &feat, &eb);
+  carve_forward(d, rows, 1, nv.in_dim, nv.out_dim, nv.ln, workspace, &f);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int64_t R = (int64_t)d->num_seeds * rows;
   if (d->reserved[0] > 0) {  // obs is uint8 [rows,H,W,C]: encode with the one-step actor's encoder (networks.py:226-227)
-    FQL_TRY(enc_forward(d, nv.enc, params, reinterpret_cast<const uint8_t*>(obs), rows, eb, feat, st));
-    obs = feat;
+    FQL_TRY(enc_forward(d, nv.enc, params, reinterpret_cast<const uint8_t*>(obs), rows, f.eb, f.feat, st));
+    obs = f.feat;
   }
-  FQL_TRY(launch_concat(obs, d->obs_dim, noise, d->action_dim, 0.f, 0, X, R, st));
+  FQL_TRY(launch_concat(obs, d->obs_dim, noise, d->action_dim, 0.f, 0, f.X, R, st));
   if (d->precision == FQL_PRECISION_BF16_TC && !tc_wide_input(d)) {
     FQL_REQUIRE(shadow != nullptr, "FQL_PRECISION_BF16_TC needs the bf16 shadow");
     const int kp = (int)round_up64(nv.in_dim, 64);
-    FQL_TRY(tc_pad_bf16(X, Xb, R, nv.in_dim, kp, st));
-    TcChainSpec t;
-    memset(&t, 0, sizeof(t));
-    t.d = d; t.L = &L; t.P = 1; t.net[0] = FQL_NET_ACTOR_ONESTEP_FLOW; t.params = params; t.shadow = shadow;
-    t.M = rows; t.X0b = Xb; t.Mcap0 = rows; t.n_steps = 1; t.out_override = actions_out; t.clip_out = 1;
-    return tc_mlp_chain(t, st);
+    FQL_TRY(tc_pad_bf16(f.X, f.Xb, R, nv.in_dim, kp, st));
+    if (d->hidden == 512) {
+      TcChainSpec t;
+      memset(&t, 0, sizeof(t));
+      t.d = d; t.L = &L; t.P = 1; t.net[0] = FQL_NET_ACTOR_ONESTEP_FLOW; t.params = params; t.shadow = shadow;
+      t.M = rows; t.X0b = f.Xb; t.Mcap0 = rows; t.n_steps = 1; t.out_override = actions_out; t.clip_out = 1;
+      return tc_mlp_chain2(t, st);
+    }
+    const TcActor t = fwd_actor(d, L, FQL_NET_ACTOR_ONESTEP_FLOW, params, shadow, rows, f);
+    return tc_actor_forward(t, actions_out, (long long)rows * d->action_dim, 1, nullptr, st);
   }
-  FQL_TRY(forward_net(d, L, FQL_NET_ACTOR_ONESTEP_FLOW, params, X, &pb, rows, st));
-  FQL_TRY(launch_clip(pb.out, actions_out, R * d->action_dim, st));
+  FQL_TRY(forward_net(d, L, FQL_NET_ACTOR_ONESTEP_FLOW, params, f.X, &f.pb, rows, st));
+  FQL_TRY(launch_clip(f.pb.out, actions_out, R * d->action_dim, st));
   return 0;
 }
 
@@ -1387,42 +1412,41 @@ extern "C" int fql_compute_flow_actions(FqlContext*, const FqlDims* d, const flo
   FQL_TRY(fql_build_layout(d, &L));
   FQL_REQUIRE(rows >= 1, "rows=%d", rows);
   const NetView& nv = L.net[FQL_NET_ACTOR_BC_FLOW];
-  float* X;
-  void* Xb;
-  void* Hx = nullptr;
-  PassBuf pb;
-  const size_t need = carve_forward(d, rows, 1, nv.in_dim, nv.out_dim, nv.ln, nullptr, &X, &pb);
+  FwdWs f;
+  const size_t need = carve_forward(d, rows, 1, nv.in_dim, nv.out_dim, nv.ln, nullptr, &f);
   FQL_REQUIRE(workspace && ws_bytes >= need, "workspace too small: have %zu need %zu", ws_bytes, need);
-  float* feat = nullptr;
-  EncBuf eb;
-  carve_forward(d, rows, 1, nv.in_dim, nv.out_dim, nv.ln, workspace, &X, &pb, &Xb, &Hx, &feat, &eb);
+  carve_forward(d, rows, 1, nv.in_dim, nv.out_dim, nv.ln, workspace, &f);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int64_t R = (int64_t)d->num_seeds * rows;
   if (d->reserved[0] > 0) {  // fql.py:162-163: encode once with actor_bc_flow_encoder, then is_encoded=True
-    FQL_TRY(enc_forward(d, nv.enc, params, reinterpret_cast<const uint8_t*>(obs), rows, eb, feat, st));
-    obs = feat;
+    FQL_TRY(enc_forward(d, nv.enc, params, reinterpret_cast<const uint8_t*>(obs), rows, f.eb, f.feat, st));
+    obs = f.feat;
   }
-  FQL_TRY(launch_concat(obs, d->obs_dim, noise, d->action_dim, 0.f, 1, X, R, st));
+  FQL_TRY(launch_concat(obs, d->obs_dim, noise, d->action_dim, 0.f, 1, f.X, R, st));
   if (d->precision == FQL_PRECISION_BF16_TC && !tc_wide_input(d)) {
     FQL_REQUIRE(shadow != nullptr, "FQL_PRECISION_BF16_TC needs the bf16 shadow");
     const int kp = (int)round_up64(nv.in_dim, 64);
-    FQL_TRY(tc_pad_bf16(X, Xb, R, nv.in_dim, kp, st));
-    if (d->hidden == 512 && Hx) {
+    FQL_TRY(tc_pad_bf16(f.X, f.Xb, R, nv.in_dim, kp, st));
+    if (d->hidden == 512) {
       TcEulerSpec e;
       memset(&e, 0, sizeof(e));
-      e.d = d; e.L = &L; e.params = params; e.shadow = shadow; e.X0b = Xb; e.Mcap0 = rows; e.r0_in = 0; e.M = rows;
-      e.a0 = noise; e.target = actions_out; e.scratch = Hx;
+      e.d = d; e.L = &L; e.params = params; e.shadow = shadow; e.X0b = f.Xb; e.Mcap0 = rows; e.r0_in = 0; e.M = rows;
+      e.a0 = noise; e.target = actions_out; e.scratch = f.Hx;
       return tc_euler_cluster(e, st);
     }
-    TcChainSpec t;
-    memset(&t, 0, sizeof(t));
-    t.d = d; t.L = &L; t.P = 1; t.net[0] = FQL_NET_ACTOR_BC_FLOW; t.params = params; t.shadow = shadow;
-    t.M = rows; t.X0b = Xb; t.Mcap0 = rows; t.n_steps = d->flow_steps; t.a0 = noise; t.target = actions_out;
-    return tc_mlp_chain(t, st);
+    // agents/fql.py:155-171: the fp32 Euler state starts as the noise; each step's last layer adds v / flow_steps to it and
+    // rewrites the action and time columns of the bf16 first-layer operand
+    FQL_CHECK_CUDA(cudaMemcpyAsync(f.act, noise, sizeof(float) * (size_t)R * d->action_dim, cudaMemcpyDeviceToDevice, st));
+    const TcActor t = fwd_actor(d, L, FQL_NET_ACTOR_BC_FLOW, params, shadow, rows, f);
+    for (int i = 0; i < d->flow_steps; i++) {
+      TcEuler eu{f.act, actions_out, i, d->flow_steps};
+      FQL_TRY(tc_actor_forward(t, nullptr, 0, 0, &eu, st));
+    }
+    return 0;
   }
   for (int i = 0; i < d->flow_steps; i++) {
-    FQL_TRY(forward_net(d, L, FQL_NET_ACTOR_BC_FLOW, params, X, &pb, rows, st));
-    FQL_TRY(launch_euler_inplace(X, pb.out, d->obs_dim, d->action_dim, R, i, d->flow_steps, actions_out, st));
+    FQL_TRY(forward_net(d, L, FQL_NET_ACTOR_BC_FLOW, params, f.X, &f.pb, rows, st));
+    FQL_TRY(launch_euler_inplace(f.X, f.pb.out, d->obs_dim, d->action_dim, R, i, d->flow_steps, actions_out, st));
   }
   return 0;
 }

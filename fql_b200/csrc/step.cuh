@@ -145,7 +145,7 @@ int launch_zero(float* p, int64_t n, cudaStream_t st);
 int launch_zero_bc(float* p, int64_t n, const int32_t* count, const FqlHparams& hp, float* bc, cudaStream_t st, int* tickets = nullptr,
                    int n_tickets = 0);
 
-// mlp_tc.cu -- tensor-core forward path
+// chain2_tc.cu -- fused per-tile MLP chains (hidden = 512): one forward pass, or the whole Euler loop, per 128-row tile and launch
 struct TcChainSpec {
   const FqlDims* d;
   const Layout* L;
@@ -166,10 +166,11 @@ struct TcChainSpec {
   const float* a0;
   float* target;
   int clip_out;
-  void* const* DGb;  // chain2 only: save bf16 gelu'(z) per hidden layer instead of the pre-activations (large-batch backward)
-  void* const* XHb;  // chain2 + LayerNorm only: save bf16 xhat per hidden layer instead of the normalised activations
-  int save_mask;     // chain2 only: bit p set = problem p writes its saves (0 = all)
+  void* const* DGb;  // optional: save bf16 gelu'(z) per hidden layer instead of the pre-activations (large-batch backward)
+  void* const* XHb;  // LayerNorm only: save bf16 xhat per hidden layer instead of the normalised activations
+  int save_mask;     // bit p set = problem p writes its saves (0 = all)
 };
+int tc_mlp_chain2(const TcChainSpec& f, cudaStream_t st);
 // chain2_tc.cu: the whole input-gradient chain of one network's backward, one launch.  Every pointer is already offset to the
 // first row of the problem; rows of group (s, e) start at ((s * ens + e) * Mcap + r0).
 struct TcChain2BwdSpec {
@@ -188,15 +189,13 @@ struct TcChain2BwdSpec {
   float* dX0;            // out (optional): fp32 [S][ens][Mcap_dz][K0] input gradient
 };
 int tc_mlp_chain2_backward(const TcChain2BwdSpec& f, cudaStream_t st);
+// mlp_tc.cu -- shared by every tensor-core MLP kernel: shape limits, bf16 shadow, padded first-layer operands, TMA tensor maps
 int tc_supported(const FqlDims* d, bool fused_kernels = true);   // fused_kernels: also the limits of the chain / cluster kernels
 inline bool tc_wide_input(const FqlDims* d) { return d->obs_dim + d->action_dim + 1 > 128; }   // pixel configs: 512 encoder features
 int64_t tc_shadow_seed_elems(const FqlDims* d, const Layout& L);
 int tc_refresh_shadow(const FqlDims* d, const Layout& L, const float* params, void* shadow, cudaStream_t st);
 int tc_refresh_shadow_lastlayer(const FqlDims* d, const Layout& L, const float* params, void* shadow, cudaStream_t st);
 int tc_pad_bf16(const float* x, void* y, int64_t rows, int K0, int K0pad, cudaStream_t st);
-int tc_mlp_chain(const TcChainSpec& f, cudaStream_t st);
-int tc_mlp_chain2_supported(const FqlDims* d);
-int tc_mlp_chain2(const TcChainSpec& f, cudaStream_t st);
 // TMA tensor maps: the driver's cuTensorMapEncodeTiled (NULL when the driver does not provide it), and a bf16 [rows][inner] row-major
 // tensor read in boxes of [box_rows][box_inner]
 PFN_cuTensorMapEncodeTiled_v12000 get_encode();

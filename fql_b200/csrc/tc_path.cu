@@ -250,7 +250,7 @@ int tc_actor_forward(const TcActor& t, float* out, long long out_ss, int clip, c
   const int H = d->hidden, NL = nv.n_layers, S = d->num_seeds;
   const int64_t seed_elems = tc_shadow_seed_elems(d, L);
   const bf16* sh = reinterpret_cast<const bf16*>(t.shadow);
-  FQL_REQUIRE(!nv.ln && nv.ens == 1, "tc_actor_forward: LayerNorm / ensemble networks use the fused chain kernel");
+  FQL_REQUIRE(!nv.ln && nv.ens == 1, "tc_actor_forward: LayerNorm / ensemble networks go through tc_critic_forward");
   for (int l = 0; l < NL; l++) {
     const bool last = (l == NL - 1);
     TcGemmSpec g;

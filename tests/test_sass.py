@@ -53,7 +53,7 @@ def _family(counts, key):
 
 
 def test_contractions_are_tcgen05_tmem_tma(sass_counts):
-    for fam in ('euler_cluster_kernel', 'mlp_chain2_kernel', 'tc_gemm_kernel', 'conv_tc_kernel', 'mlp_chain_tc_kernel'):
+    for fam in ('euler_cluster_kernel', 'mlp_chain2_kernel', 'tc_gemm_kernel', 'conv_tc_kernel'):
         ks = _family(sass_counts, fam)
         assert ks, fam
         for name, c in ks.items():
@@ -61,6 +61,6 @@ def test_contractions_are_tcgen05_tmem_tma(sass_counts):
 
 
 def test_single_thread_roles_are_warp_uniform(sass_counts):
-    for fam in ('euler_cluster_kernel', 'mlp_chain2_kernel', 'tc_gemm_kernel', 'conv_tc_kernel', 'mlp_chain_tc_kernel'):
+    for fam in ('euler_cluster_kernel', 'mlp_chain2_kernel', 'tc_gemm_kernel', 'conv_tc_kernel'):
         for name, c in _family(sass_counts, fam).items():
             assert c['bcast'] <= max(12, c['mma'] // 4), (name, c)

@@ -653,7 +653,7 @@ CHAIN_TOL_SAMPLE, CHAIN_TOL_FLOW = 1e-2, 3e-3
 @pytest.mark.parametrize('pseed', [0, 1])
 @pytest.mark.parametrize('rows', [1, 127, 128, 129, 1000, 6144])
 def test_forward_chains_same_rounding(rows, pseed, env, monkeypatch):
-    """fql_sample_actions (chain kernel, mlp_tc.cu) and fql_compute_flow_actions (cluster Euler kernel at hidden 512,
+    """fql_sample_actions (chain kernel, chain2_tc.cu) and fql_compute_flow_actions (cluster Euler kernel at hidden 512,
     euler_cluster.cu) per row against the fp64 oracle with the kernels' storage rounding: bf16 weights and layer inputs, fp32
     Euler state, bf16 action / time columns.  The stand-alone entry points choose their kernel from the hidden width alone, so the
     6144-row case (48 row tiles, where the step switches to the per-tile chain kernels) and FQL_B200_CHAIN_MIN_TILES run the same

@@ -1,5 +1,5 @@
 """FQL_PRECISION_BF16_TC at the sizes north_star names (BASELINE configs 3 and 4), where the large-batch routing is reached
-naturally: per-tile fused chain kernels (seeds x 128-row tiles >= 48), multi-CTA loss reductions with atomics, two-stage column
+naturally: per-tile fused chain kernels (hidden 512, seeds x 128-row tiles >= 48), multi-CTA loss reductions with atomics, two-stage column
 sums, and the clusters-of-8 fallback of the cluster kernels (more row tiles than the GPU holds clusters of 16).
 
 The fp64 oracle cannot run 16384 rows in seconds, so the batch is R copies of one 256-row block: every loss is a batch mean, so
@@ -30,11 +30,13 @@ def _check(agent, agent_cfg, info, state, new_state, ref_info, ref_grads, what):
     print(f'{what}: worst grad err {worst:.2e}, worst update err {d:.2e}')
 
 
-@pytest.mark.parametrize('B,block', [(8192, 256), (16384, 256), (1000, 250)], ids=['B8192', 'B16384', 'B1000-ragged-nc8'])
-def test_tc_large_batch_update(B, block):
-    """humanoidmaze-medium shape (config 3).  B=1000 = 7 full tiles + 104 rows: 8 row tiles > 7 clusters of 16 -> clusters of 8."""
+@pytest.mark.parametrize('B,block,hidden', [(8192, 256, 512), (16384, 256, 512), (1000, 250, 512), (6144, 256, 256)],
+                         ids=['B8192', 'B16384', 'B1000-ragged-nc8', 'B6144-h256'])
+def test_tc_large_batch_update(B, block, hidden):
+    """humanoidmaze-medium shape (config 3).  B=1000 = 7 full tiles + 104 rows: 8 row tiles > 7 clusters of 16 -> clusters of 8.
+    hidden=256 at 48 row tiles: the fused chains are hidden-512 only, so the whole step runs layer by layer through tc_gemm at large M."""
     F, A = 69, 21
-    cfg, state, batch, noise = make_case(dict(discount=0.995, alpha=30.0), block, F, A, seed=B % 997, hidden=512)
+    cfg, state, batch, noise = make_case(dict(discount=0.995, alpha=30.0), block, F, A, seed=B % 997, hidden=hidden)
     new_state, ref_info, ref_grads = O.update(copy.deepcopy(state), cfg, batch, noise)
     rep = B // block
     big_b = {k: np.concatenate([v] * rep, 0) for k, v in batch.items()}
