@@ -69,6 +69,18 @@ class FqlTestGemm(C.Structure):
                 [(n, C.c_int32) for n in ('F', 'Adim', 'step', 'n_steps', 'clip')])
 
 
+class FqlTestConv(C.Structure):
+    _fields_ = ([(n, C.c_int32) for n in ('mode', 'B', 'H', 'W', 'cin', 'cin_p', 'cout')] + [('scale', C.c_float)] +
+                [(n, C.c_void_p) for n in ('w', 'x', 'dy', 'bias', 'mask', 'add')] + [('relu_out', C.c_int32)] +
+                [(n, C.c_void_p) for n in ('out', 'out_relu', 'gw', 'gb', 'workspace')] + [('ws_bytes', C.c_size_t)])
+
+
+TEST_CONV_FWD, TEST_CONV_DGRAD, TEST_CONV_WGRAD = 0, 1, 2
+# fql_test_encoder_bf16 offsets[]: byte offsets of the carved buffers (FQL_TEST_ENC_* of include/fql_b200.h), then the workspace size
+TEST_ENC_BUFS = ('img', 'y0', 'p0', 'p1', 'p2', 'r1_0', 'r1_1', 'r1_2', 'r2_0', 'r2_1', 'r2_2', 'xs0', 'xs1', 'xs2', 'arg0', 'arg1', 'arg2',
+                 'flat', 'z', 'dz', 'dzb', 'dflat', 'wf', 'wd', 'wdense')
+TEST_ENC_NOFF = len(TEST_ENC_BUFS) + 1
+
 TC_MODE_STORE_F32, TC_MODE_FWD_HIDDEN, TC_MODE_DGRAD_GELU, TC_MODE_EULER, TC_MODE_WGRAD_LN = 0, 1, 2, 3, 4
 
 
@@ -115,6 +127,11 @@ _SIGS = {
                                          C.c_int64, C.c_int64, C.c_void_p]),
     'fql_test_colsum_bf16': (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_int64, C.c_int32, C.c_int64,
                                        C.c_void_p]),
+    'fql_test_pool_bf16': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    'fql_test_pool_bwd_bf16': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    'fql_test_conv_bf16': (C.c_int, [C.POINTER(FqlTestConv), C.c_void_p]),
+    'fql_test_encoder_bf16': (C.c_int, [C.POINTER(FqlDims), C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_size_t, C.POINTER(C.c_int64), C.c_void_p]),
     'fql_set_early_grads_event':(C.c_int, [C.c_void_p, C.c_void_p]),
     'fql_early_grads_floats': (C.c_int64, [C.POINTER(FqlDims)]),
     'fql_total_loss': (C.c_int, [C.c_void_p, C.POINTER(FqlDims), C.POINTER(FqlHparams), C.POINTER(FqlBatch), C.POINTER(FqlState),

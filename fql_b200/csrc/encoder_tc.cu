@@ -943,3 +943,96 @@ extern "C" int fql_conv3x3_wgrad_bf16(const void* x, const void* dy, int32_t B, 
   return conv_wgrad_tc(reinterpret_cast<const bf16*>(x), cin, cin, cout, reinterpret_cast<const bf16*>(dy), B, H, W, 1.0f, partial, gw, gb,
                        reinterpret_cast<cudaStream_t>(stream));
 }
+
+// ---------------------------------------------------------------------------------------------------------------
+// Test hooks (include/fql_b200.h): the pooling kernels, one convolution with every argument the encoder passes use, and a whole
+// encoder pass whose saved activations the caller can read back -- each launched exactly as enc_tc_forward / enc_tc_backward launch
+// them, so that tests/test_encoder_tc_kernels_gpu.py can check every kernel of this file against a reference on its own.
+// ---------------------------------------------------------------------------------------------------------------
+extern "C" int fql_test_pool_bf16(const void* in, void* out, void* out_relu, void* arg, int32_t B, int32_t H, int32_t W, int32_t C, void* stream) {
+  FQL_REQUIRE(in && out && out_relu && arg, "fql_test_pool_bf16: NULL argument");
+  FQL_REQUIRE(B >= 1 && H >= 1 && W >= 1 && C >= 8 && C % 8 == 0, "fql_test_pool_bf16: B=%d H=%d W=%d C=%d (C must be a multiple of 8)", B, H, W, C);
+  const long long Ho = (H + 1) / 2, Wo = (W + 1) / 2;
+  return launch1d(pool_fwd_bf16_kernel, B * Ho * Wo * (C / 8), reinterpret_cast<cudaStream_t>(stream), reinterpret_cast<const bf16*>(in),
+                  reinterpret_cast<bf16*>(out), reinterpret_cast<bf16*>(out_relu), reinterpret_cast<uint8_t*>(arg), (long long)B, H, W, C);
+}
+
+extern "C" int fql_test_pool_bwd_bf16(const void* dout, const void* arg, void* din, int32_t B, int32_t H, int32_t W, int32_t C, void* stream) {
+  FQL_REQUIRE(dout && arg && din, "fql_test_pool_bwd_bf16: NULL argument");
+  FQL_REQUIRE(B >= 1 && H >= 1 && W >= 1 && C >= 8 && C % 8 == 0, "fql_test_pool_bwd_bf16: B=%d H=%d W=%d C=%d (C must be a multiple of 8)", B, H, W, C);
+  return launch1d(pool_bwd_bf16_kernel, (long long)B * H * W * (C / 8), reinterpret_cast<cudaStream_t>(stream), reinterpret_cast<const bf16*>(dout),
+                  reinterpret_cast<const uint8_t*>(arg), reinterpret_cast<bf16*>(din), (long long)B, H, W, C);
+}
+
+extern "C" int fql_test_conv_bf16(const FqlTestConv* c, void* stream) {
+  FQL_REQUIRE(c != nullptr, "fql_test_conv_bf16: spec is NULL");
+  FQL_REQUIRE(c->workspace && c->ws_bytes >= fql_conv3x3_workspace_bytes(), "fql_test_conv_bf16: workspace NULL / too small");
+  FQL_REQUIRE(c->B >= 1 && c->H >= 1 && c->W >= 1 && c->cin >= 1 && c->cin <= c->cin_p && (c->cin_p == 16 || c->cin_p == 32) &&
+                  (c->cout == 16 || c->cout == 32),
+              "fql_test_conv_bf16: B=%d H=%d W=%d cin=%d cin_p=%d cout=%d", c->B, c->H, c->W, c->cin, c->cin_p, c->cout);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  bf16* wf = reinterpret_cast<bf16*>(c->workspace);
+  bf16* wd = wf + 9 * WSLOT;
+  if (c->mode == FQL_TEST_CONV_WGRAD) {
+    FQL_REQUIRE(c->x && c->dy && c->gw && c->gb, "fql_test_conv_bf16: the weight gradient needs x, dy, gw and gb");
+    float* partial = reinterpret_cast<float*>(reinterpret_cast<char*>(c->workspace) + (size_t)2 * 9 * WSLOT * 2);
+    return conv_wgrad_tc(reinterpret_cast<const bf16*>(c->x), c->cin_p, c->cin, c->cout, reinterpret_cast<const bf16*>(c->dy), c->B, c->H, c->W,
+                         c->scale, partial, c->gw, c->gb, st);
+  }
+  FQL_REQUIRE(c->mode == FQL_TEST_CONV_FWD || c->mode == FQL_TEST_CONV_DGRAD, "fql_test_conv_bf16: mode %d", c->mode);
+  FQL_REQUIRE(c->w && c->x && c->out, "fql_test_conv_bf16: NULL w / x / out");
+  FQL_REQUIRE(c->mode == FQL_TEST_CONV_FWD || c->cin == c->cin_p, "fql_test_conv_bf16: the input gradient needs cin == cin_p");
+  PrepArgs pa;
+  memset(&pa, 0, sizeof(pa));
+  pa.job[0].off_w = 0; pa.job[0].cin = c->cin; pa.job[0].cin_p = c->cin_p; pa.job[0].cout = c->cout;
+  enc_prep_weights_kernel<<<dim3(16, 18), 256, 0, st>>>(c->w, pa, wf, wd, nullptr);
+  FQL_CHECK_LAUNCH();
+  const bool fwd = c->mode == FQL_TEST_CONV_FWD;
+  return conv_tc(reinterpret_cast<const bf16*>(c->x), fwd ? c->cin_p : c->cout, fwd ? c->cout : c->cin, fwd ? wf : wd, c->B, c->H, c->W, c->scale,
+                 c->bias, reinterpret_cast<const bf16*>(c->mask), reinterpret_cast<const bf16*>(c->add), c->relu_out,
+                 reinterpret_cast<bf16*>(c->out), reinterpret_cast<bf16*>(c->out_relu), st);
+}
+
+extern "C" int fql_test_encoder_bf16(const FqlDims* d, int32_t net, const float* params, const uint8_t* obs, int32_t B, const float* dfeat,
+                                     float* feat, float* grads, void* workspace, size_t ws_bytes, int64_t* offsets, void* stream) {
+  FQL_REQUIRE(d && offsets, "fql_test_encoder_bf16: NULL dims / offsets");
+  FQL_REQUIRE(net >= 0 && net < FQL_NUM_NETS && B >= 1, "fql_test_encoder_bf16: net %d, B %d", net, B);
+  Layout L;
+  FQL_TRY(fql_build_layout(d, &L));
+  FQL_REQUIRE(L.net[net].has_enc, "fql_test_encoder_bf16: network %d has no encoder (dims without an image)", net);
+  const bool bwd = dfeat != nullptr;
+  EncBuf e;
+  memset(&e, 0, sizeof(e));
+  const size_t need = enc_tc_carve(d, B, nullptr, &e, bwd);
+  offsets[FQL_TEST_ENC_NOFF - 1] = (int64_t)need;
+  if (!workspace) return 0;
+  FQL_REQUIRE(ws_bytes >= need && (reinterpret_cast<uintptr_t>(workspace) & 255) == 0,
+              "fql_test_encoder_bf16: workspace %zu bytes (needs %zu, 256-byte aligned)", ws_bytes, need);
+  FQL_REQUIRE(params && obs && feat && (!bwd || grads), "fql_test_encoder_bf16: NULL params / obs / feat / grads");
+  enc_tc_carve(d, B, workspace, &e, bwd);
+  const char* base = reinterpret_cast<const char*>(workspace);
+  auto at = [&](int k, const void* p) { offsets[k] = p ? (int64_t)(reinterpret_cast<const char*>(p) - base) : -1; };
+  const EncTc& t = e.tc;
+  at(FQL_TEST_ENC_IMG, t.img);
+  at(FQL_TEST_ENC_Y0, t.y0);
+  for (int i = 0; i < 3; i++) {
+    at(FQL_TEST_ENC_P + i, t.p[i]);
+    at(FQL_TEST_ENC_R1 + i, t.r1[i]);
+    at(FQL_TEST_ENC_R2 + i, t.r2[i]);
+    at(FQL_TEST_ENC_XS + i, t.xs[i]);
+    at(FQL_TEST_ENC_ARG + i, e.arg[i]);
+  }
+  at(FQL_TEST_ENC_FLAT, t.flat);
+  at(FQL_TEST_ENC_Z, e.z);
+  at(FQL_TEST_ENC_DZ, e.dz);
+  at(FQL_TEST_ENC_DZB, t.dzb);
+  at(FQL_TEST_ENC_DFLAT, e.dflat);
+  at(FQL_TEST_ENC_WF, t.wf);
+  at(FQL_TEST_ENC_WD, t.wd);
+  at(FQL_TEST_ENC_WDENSE, t.wdense);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  const EncView& v = L.net[net].enc;
+  FQL_TRY(enc_tc_forward(d, v, params, obs, B, e, feat, st));
+  if (bwd) FQL_TRY(enc_tc_backward(d, v, params, grads, obs, B, e, dfeat, st));
+  return 0;
+}

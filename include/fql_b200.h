@@ -270,6 +270,42 @@ int fql_test_gelu_bwd_bf16(const float* dH, const float* Z, float* dZ, void* dZb
 int fql_test_colsum_bf16(const void* X, int64_t G, int64_t M, int32_t N, float* out, int64_t out_stride_g0, int32_t G0,
                          int64_t out_stride_g1, void* stream);
 
+/* ---- test hooks: the tensor-core ImpalaEncoder of FQL_PRECISION_BF16_ENC / _TC (fql_b200/csrc/encoder_tc.cu) ------------------------
+ * Each launches its kernels exactly as the encoder passes of the step do; nothing here is used by the step.  bf16 tensors are NHWC. */
+/* max_pool 3x3/2 SAME: in [B,H,W,C] -> out, out_relu = max(out, 0) and arg (uint8 ky * 3 + kx of the first maximum) [B,Ho,Wo,C],
+ * Ho = (H + 1) / 2.  C % 8 == 0. */
+int fql_test_pool_bf16(const void* in, void* out, void* out_relu, void* arg, int32_t B, int32_t H, int32_t W, int32_t C, void* stream);
+/* its gradient: din [B,H,W,C] = sum over the windows whose argmax points at the pixel of dout [B,Ho,Wo,C] */
+int fql_test_pool_bwd_bf16(const void* dout, const void* arg, void* din, int32_t B, int32_t H, int32_t W, int32_t C, void* stream);
+enum { FQL_TEST_CONV_FWD = 0, FQL_TEST_CONV_DGRAD = 1, FQL_TEST_CONV_WGRAD = 2 };
+typedef struct FqlTestConv {    /* one 3x3 SAME convolution with the HWIO kernel w [3,3,cin,cout] (fp32, rounded to bf16 operands) */
+  int32_t mode;                 /* FQL_TEST_CONV_*                                                                                */
+  int32_t B, H, W;
+  int32_t cin, cin_p, cout;     /* cin: real input channels of w; cin_p (>= cin): channels of the activation tensor (16 for frames) */
+  float scale;                  /* FWD: out = epilogue(scale * acc + bias); WGRAD: gw = scale * sum (gb is not scaled)              */
+  const float* w;               /* FWD / DGRAD                                                                                    */
+  const void* x;                /* FWD / WGRAD: bf16 [B,H,W,cin_p]; DGRAD: dY bf16 [B,H,W,cout]                                   */
+  const void* dy;               /* WGRAD: bf16 [B,H,W,cout]                                                                       */
+  const float* bias;            /* FWD / DGRAD epilogue: v = scale * acc + bias; v = mask > 0 ? v : 0; v += add; relu_out: relu(v) */
+  const void *mask, *add;
+  int32_t relu_out;
+  void *out, *out_relu;         /* bf16 [B,H,W,cout] (DGRAD: [B,H,W,cin]); out_relu (optional) = relu(v) before relu_out          */
+  float *gw, *gb;               /* WGRAD: fp32 [3,3,cin,cout] and [cout]                                                          */
+  void* workspace;              /* fql_conv3x3_workspace_bytes() bytes                                                            */
+  size_t ws_bytes;
+} FqlTestConv;
+int fql_test_conv_bf16(const FqlTestConv* c, void* stream);
+/* One encoder forward (and, with dfeat != NULL, backward) of network `net` over B frames obs uint8 [B,img_h,img_w,img_c]:
+ * feat [B,512] = encoder(obs); grads receives d(dfeat . feat)/d(encoder leaves) at the arena offsets of fql_layout (nothing else of
+ * grads is written).  offsets[FQL_TEST_ENC_NOFF] receives the byte offset inside workspace of every buffer the pass carves, in the
+ * order of FQL_TEST_ENC_* (-1 = not carved), and offsets[FQL_TEST_ENC_NOFF - 1] the workspace bytes it needs; with workspace == NULL
+ * only that size is written.  workspace must be 256-byte aligned. */
+enum { FQL_TEST_ENC_IMG = 0, FQL_TEST_ENC_Y0 = 1, FQL_TEST_ENC_P = 2, FQL_TEST_ENC_R1 = 5, FQL_TEST_ENC_R2 = 8, FQL_TEST_ENC_XS = 11,
+       FQL_TEST_ENC_ARG = 14, FQL_TEST_ENC_FLAT = 17, FQL_TEST_ENC_Z = 18, FQL_TEST_ENC_DZ = 19, FQL_TEST_ENC_DZB = 20,
+       FQL_TEST_ENC_DFLAT = 21, FQL_TEST_ENC_WF = 22, FQL_TEST_ENC_WD = 23, FQL_TEST_ENC_WDENSE = 24, FQL_TEST_ENC_NOFF = 26 };
+int fql_test_encoder_bf16(const FqlDims* d, int32_t net, const float* params, const uint8_t* obs, int32_t B, const float* dfeat, float* feat,
+                          float* grads, void* workspace, size_t ws_bytes, int64_t* offsets, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
