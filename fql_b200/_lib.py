@@ -16,7 +16,7 @@ NUM_RAW = 16
 NET_NAMES = ('actor_bc_flow', 'actor_onestep_flow', 'critic', 'target_critic')
 NET_ACTOR_BC_FLOW, NET_ACTOR_ONESTEP_FLOW, NET_CRITIC, NET_TARGET_CRITIC = 0, 1, 2, 3
 LEAF_KINDS = ('kernel', 'bias', 'scale', 'bias', 'kernel', 'bias', 'kernel', 'bias')
-PRECISION_FP32, PRECISION_BF16_TC, PRECISION_BF16_ENC = 0, 1, 2
+PRECISION_FP32, PRECISION_BF16_TC, PRECISION_BF16_ENC, PRECISION_FP32_TC = 0, 1, 2, 3
 
 
 class FqlDims(C.Structure):
@@ -69,6 +69,15 @@ class FqlTestGemm(C.Structure):
                 [(n, C.c_int32) for n in ('F', 'Adim', 'step', 'n_steps', 'clip')])
 
 
+class FqlTestGPtr(C.Structure):
+    _fields_ = [('base', C.c_void_p * 3), ('stride_s', C.c_int64), ('stride_e', C.c_int64)]
+
+
+class FqlTestGemmF32(C.Structure):
+    _fields_ = ([(n, C.c_int32) for n in ('M', 'N', 'K', 'P', 'S', 'E', 'lda', 'ldb', 'ldo', 'ld_pre', 'ld_mulz', 'trans_a', 'trans_b',
+                                          'act_gelu')] + [(n, FqlTestGPtr) for n in ('A', 'B', 'bias', 'mulz', 'out_pre', 'out')])
+
+
 class FqlTestConv(C.Structure):
     _fields_ = ([(n, C.c_int32) for n in ('mode', 'B', 'H', 'W', 'cin', 'cin_p', 'cout')] + [('scale', C.c_float)] +
                 [(n, C.c_void_p) for n in ('w', 'x', 'dy', 'bias', 'mask', 'add')] + [('relu_out', C.c_int32)] +
@@ -119,6 +128,7 @@ _SIGS = {
     'fql_conv3x3_wgrad_bf16': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p,
                                          C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     'fql_test_tc_gemm': (C.c_int, [C.POINTER(FqlTestGemm), C.c_void_p]),
+    'fql_test_gemm_f32': (C.c_int, [C.POINTER(FqlTestGemmF32), C.c_int32, C.c_void_p]),
     'fql_test_act_ln_bf16': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     'fql_test_ln_bwd_bf16': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32,

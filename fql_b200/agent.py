@@ -156,8 +156,13 @@ class FQLAgent:
         if world_size is not None:
             self.world = int(world_size)  # explicit override: the caller drives grads_phase / apply_phase itself
         # 'bf16': every contraction on tcgen05 (pixel configs: implicit-GEMM encoders + layer-by-layer MLPs); 'bf16-enc' (pixel
-        # configs only): tcgen05 encoders, the MLPs behind them in fp32
-        self._precision = {'fp32': _lib.PRECISION_FP32, 'bf16': _lib.PRECISION_BF16_TC, 'bf16-enc': _lib.PRECISION_BF16_ENC}[precision]
+        # configs only): tcgen05 encoders, the MLPs behind them in fp32; 'fp32-tc' (state observations only): the fp32 schedule with
+        # every Dense contraction on tcgen05 as 3xTF32, at the fp32 parity tolerance
+        self._precision = {'fp32': _lib.PRECISION_FP32, 'bf16': _lib.PRECISION_BF16_TC, 'bf16-enc': _lib.PRECISION_BF16_ENC,
+                           'fp32-tc': _lib.PRECISION_FP32_TC}[precision]
+        if self._precision == _lib.PRECISION_FP32_TC and cfg.get('encoder') is not None:
+            raise NotImplementedError("precision='fp32-tc' supports state observations only (no tf32 convolutions); "
+                                      "use 'fp32' or 'bf16' with encoder='impala_small'")
         self._hidden, self._num_hidden = ah[0], len(ah)
         self._image = ob_dims if cfg.get('encoder') is not None else None
         self._feat = 512 if self._image else ob_dims[0]

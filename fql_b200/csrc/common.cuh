@@ -135,8 +135,10 @@ struct GemmArgs {
   int act_gelu;           // out = gelu(acc+bias)
   int S, E;               // seeds, heads (groups = P*S*E)
   int P;
+  int tf32x3;             // FQL_PRECISION_FP32_TC: 3xTF32 on tcgen05 (gemm_tf32x3.cu) instead of FFMA
 };
 int launch_gemm(const GemmArgs& a, cudaStream_t st);
+int launch_gemm_tf32x3(const GemmArgs& a, cudaStream_t st);
 
 // rows kernel: H = LN(gelu(Z)) (or just gelu), per group scale/bias
 struct ActLnArgs {

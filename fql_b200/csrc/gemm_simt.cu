@@ -268,6 +268,7 @@ __global__ void colsum_final_kernel(ColSumArgs a, const float* __restrict__ part
 }  // namespace
 
 int launch_gemm(const GemmArgs& a, cudaStream_t st) {
+  if (a.tf32x3) return launch_gemm_tf32x3(a, st);
   if (a.M <= 0 || a.N <= 0) return 0;
   const int G = a.P * a.S * a.E;
   const int64_t big_tiles = (int64_t)((a.M + 63) / 64) * ((a.N + 63) / 64) * G;

@@ -40,8 +40,12 @@ int fql_validate_dims(const FqlDims* d) {
   FQL_REQUIRE(d->hidden >= 1 && d->num_hidden >= 1 && d->num_hidden + 1 <= FQL_MAXL, "hidden=%d num_hidden=%d", d->hidden, d->num_hidden);
   FQL_REQUIRE(d->num_seeds >= 1, "num_seeds=%d", d->num_seeds);
   FQL_REQUIRE(d->flow_steps >= 1, "flow_steps=%d", d->flow_steps);
-  FQL_REQUIRE(d->precision == FQL_PRECISION_FP32 || d->precision == FQL_PRECISION_BF16_TC || d->precision == FQL_PRECISION_BF16_ENC,
+  FQL_REQUIRE(d->precision == FQL_PRECISION_FP32 || d->precision == FQL_PRECISION_BF16_TC || d->precision == FQL_PRECISION_BF16_ENC ||
+                  d->precision == FQL_PRECISION_FP32_TC,
               "precision=%d", d->precision);
+  // the encoders pick their tensor-core path for any precision other than FP32; this mode has no tf32 convolutions
+  FQL_REQUIRE(d->precision != FQL_PRECISION_FP32_TC || d->reserved[0] == 0,
+              "FQL_PRECISION_FP32_TC ('fp32-tc') is a state-observation mode: pixel configs (encoder='impala_small') are not supported");
   FQL_REQUIRE(d->precision != FQL_PRECISION_BF16_ENC || d->reserved[0] > 0, "FQL_PRECISION_BF16_ENC is a pixel-config mode (encoder='impala_small')");
   if (d->reserved[0] > 0) {  // pixel observations through ImpalaEncoder('impala_small')
     FQL_REQUIRE(d->reserved[1] > 0 && d->reserved[2] > 0 && d->reserved[2] <= 32, "image dims %dx%dx%d", d->reserved[0], d->reserved[1], d->reserved[2]);
@@ -254,6 +258,7 @@ struct FwdSpec {
   PassBuf* buf;
   int r0;
   int save_z;
+  int tf32x3;       // FQL_PRECISION_FP32_TC: the GEMMs on the 3xTF32 tensor-core kernel
 };
 
 int mlp_forward(const FwdSpec& f, cudaStream_t st) {
@@ -288,6 +293,7 @@ int mlp_forward(const FwdSpec& f, cudaStream_t st) {
       }
     }
     a.act_gelu = (!last && !n0.ln) ? 1 : 0;
+    a.tf32x3 = f.tf32x3;
     FQL_TRY(launch_gemm(a, st));
     if (!last && n0.ln) {
       ActLnArgs r;
@@ -327,6 +333,7 @@ struct BwdSpec {
   const float* dOut;  // [S][E][M][out_dim]
   float* dpp[2];      // [S][E][M][H]
   float* dX0;         // optional [S][E][M][K0]
+  int tf32x3;         // FQL_PRECISION_FP32_TC: the GEMMs on the 3xTF32 tensor-core kernel
 };
 
 int mlp_backward(const BwdSpec& b, cudaStream_t st) {
@@ -349,6 +356,7 @@ int mlp_backward(const BwdSpec& b, cudaStream_t st) {
       else { a.A.base[0] = b.buf->Hh[l - 1] + goff_rows * b.H; a.A.stride_s = (int64_t)b.E * Mcap * b.H; a.A.stride_e = Mcap * b.H; a.lda = b.H; }
       a.B.base[0] = dZ; a.B.stride_s = dz_ss; a.B.stride_e = dz_se; a.ldb = ldz;
       a.out.base[0] = b.grads + n.off_w[l]; a.out.stride_s = b.arena; a.out.stride_e = (int64_t)K * N; a.ldo = N;
+      a.tf32x3 = b.tf32x3;
       FQL_TRY(launch_gemm(a, st));
       ColSumArgs c;  // db[N] = sum_rows dZ
       memset(&c, 0, sizeof(c));
@@ -364,6 +372,7 @@ int mlp_backward(const BwdSpec& b, cudaStream_t st) {
     a.A.base[0] = dZ; a.A.stride_s = dz_ss; a.A.stride_e = dz_se; a.lda = ldz;
     a.trans_b = 1;
     a.B.base[0] = b.params + n.off_w[l]; a.B.stride_s = b.arena; a.B.stride_e = (int64_t)K * N; a.ldb = N;
+    a.tf32x3 = b.tf32x3;
     if (l == 0) {
       a.out.base[0] = b.dX0; a.out.stride_s = (int64_t)b.E * b.M * K; a.out.stride_e = (int64_t)b.M * K; a.ldo = K;
       FQL_TRY(launch_gemm(a, st));
@@ -1011,6 +1020,7 @@ int enqueue_step(FqlContext* ctx, const StepCall& c, cudaStream_t S0) {
   const StepShape sh = make_shape(c.d);
   const FqlHparams hp = *c.hp;
   const int S = sh.S, B = sh.B, H = sh.H;
+  const int x3 = c.d->precision == FQL_PRECISION_FP32_TC;
   FQL_REQUIRE(!(c.d->normalize_q_loss && c.d->global_batch != c.d->batch) || ctx->dp.active,
               "normalize_q_loss with a data-parallel split needs the global mean|q| inside the step (agents/fql.py:74-76): attach a peer-memory "
               "communicator (fql_dp_attach); the fql_step_grads / fql_step_apply split cannot provide it");
@@ -1037,6 +1047,7 @@ int enqueue_step(FqlContext* ctx, const StepCall& c, cudaStream_t S0) {
     // ---- S1: bc-flow network on {BC rows, Euler rows}, then the Euler chain
     FwdSpec fF;
     memset(&fF, 0, sizeof(fF));
+    fF.tf32x3 = x3;
     fF.P = 1; fF.nv[0] = &L.net[FQL_NET_ACTOR_BC_FLOW]; fF.params = P; fF.arena = L.arena;
     fF.S = S; fF.E = 1; fF.M = 2 * B; fF.H = H; fF.X0 = w.XF; fF.Mcap0 = 2 * B; fF.r0_in = 0;
     fF.buf = &w.pF; fF.r0 = 0; fF.save_z = 1;
@@ -1054,6 +1065,7 @@ int enqueue_step(FqlContext* ctx, const StepCall& c, cudaStream_t S0) {
     // ---- S0: one-step actor, then the grouped critic pass
     FwdSpec fO;
     memset(&fO, 0, sizeof(fO));
+    fO.tf32x3 = x3;
     fO.P = 1; fO.nv[0] = &L.net[FQL_NET_ACTOR_ONESTEP_FLOW]; fO.params = P; fO.arena = L.arena;
     fO.S = S; fO.E = 1; fO.M = 3 * B; fO.H = H; fO.X0 = w.XO; fO.Mcap0 = 3 * B; fO.r0_in = 0;
     fO.buf = &w.pO; fO.r0 = 0; fO.save_z = 1;
@@ -1061,6 +1073,7 @@ int enqueue_step(FqlContext* ctx, const StepCall& c, cudaStream_t S0) {
     FQL_TRY(launch_post_onestep(sh, b, w, raw, S0));
     FwdSpec fC;
     memset(&fC, 0, sizeof(fC));
+    fC.tf32x3 = x3;
     fC.P = 3; fC.nv[0] = &L.net[FQL_NET_TARGET_CRITIC]; fC.nv[1] = &L.net[FQL_NET_CRITIC]; fC.nv[2] = &L.net[FQL_NET_CRITIC];
     fC.params = P; fC.arena = L.arena; fC.S = S; fC.E = 2; fC.M = B; fC.H = H; fC.X0 = w.XC; fC.Mcap0 = B; fC.r0_in = 0;
     fC.buf = &w.pC; fC.r0 = 0; fC.save_z = 1;
@@ -1077,6 +1090,7 @@ int enqueue_step(FqlContext* ctx, const StepCall& c, cudaStream_t S0) {
     if (c.do_backward) {
       BwdSpec bF;
       memset(&bF, 0, sizeof(bF));
+      bF.tf32x3 = x3;
       bF.nv = &L.net[FQL_NET_ACTOR_BC_FLOW]; bF.params = P; bF.grads = c.st->grads; bF.arena = L.arena;
       bF.S = S; bF.E = 1; bF.M = B; bF.H = H; bF.X0 = w.XF; bF.Mcap0 = 2 * B; bF.buf = &w.pF; bF.p = 0; bF.r0 = 0;
       bF.dOut = w.dpred; bF.dpp[0] = w.dF[0]; bF.dpp[1] = w.dF[1];
@@ -1086,6 +1100,7 @@ int enqueue_step(FqlContext* ctx, const StepCall& c, cudaStream_t S0) {
       FQL_CHECK_CUDA(cudaStreamWaitEvent(S2, ev_cpost, 0));
       BwdSpec bC;
       memset(&bC, 0, sizeof(bC));
+      bC.tf32x3 = x3;
       bC.nv = &L.net[FQL_NET_CRITIC]; bC.params = P; bC.grads = c.st->grads; bC.arena = L.arena;
       bC.S = S; bC.E = 2; bC.M = B; bC.H = H; bC.X0 = w.XC + (int64_t)1 * S * B * (sh.F + sh.A); bC.Mcap0 = B;
       bC.buf = &w.pC; bC.p = 1; bC.r0 = 0; bC.dOut = w.dq; bC.dpp[0] = w.dC[0]; bC.dpp[1] = w.dC[1];
@@ -1100,6 +1115,7 @@ int enqueue_step(FqlContext* ctx, const StepCall& c, cudaStream_t S0) {
     if (c.do_backward) {
       BwdSpec bQ;
       memset(&bQ, 0, sizeof(bQ));
+      bQ.tf32x3 = x3;
       bQ.nv = &L.net[FQL_NET_CRITIC]; bQ.params = P; bQ.grads = nullptr; bQ.arena = L.arena;
       bQ.S = S; bQ.E = 2; bQ.M = B; bQ.H = H; bQ.X0 = w.XC + (int64_t)2 * S * B * (sh.F + sh.A); bQ.Mcap0 = B;
       bQ.buf = &w.pC; bQ.p = 2; bQ.r0 = 0; bQ.dOut = w.dqs; bQ.dpp[0] = w.dCp[0]; bQ.dpp[1] = w.dCp[1]; bQ.dX0 = w.dX0;
@@ -1110,6 +1126,7 @@ int enqueue_step(FqlContext* ctx, const StepCall& c, cudaStream_t S0) {
     if (c.do_backward) {
       BwdSpec bO;
       memset(&bO, 0, sizeof(bO));
+      bO.tf32x3 = x3;
       bO.nv = &L.net[FQL_NET_ACTOR_ONESTEP_FLOW]; bO.params = P; bO.grads = c.st->grads; bO.arena = L.arena;
       bO.S = S; bO.E = 1; bO.M = B; bO.H = H; bO.X0 = w.XO + (int64_t)B * (sh.F + sh.A); bO.Mcap0 = 3 * B;
       bO.buf = &w.pO; bO.p = 0; bO.r0 = B; bO.dOut = w.dapi; bO.dpp[0] = w.dO[0]; bO.dpp[1] = w.dO[1];
@@ -1347,6 +1364,7 @@ static int forward_net(const FqlDims* d, const Layout& L, int net, const float* 
   memset(&f, 0, sizeof(f));
   f.P = 1; f.nv[0] = &L.net[net]; f.params = params; f.arena = L.arena;
   f.S = d->num_seeds; f.E = L.net[net].ens; f.M = rows; f.H = d->hidden; f.X0 = X; f.Mcap0 = rows; f.buf = pb;
+  f.tf32x3 = d->precision == FQL_PRECISION_FP32_TC;
   return mlp_forward(f, st);
 }
 
@@ -1355,7 +1373,7 @@ extern "C" int fql_mlp_forward(FqlContext*, const FqlDims* d, int32_t net, const
   Layout L;
   FQL_TRY(fql_build_layout(d, &L));
   FQL_REQUIRE(net >= 0 && net < FQL_NUM_NETS && rows >= 1, "bad net/rows");
-  FQL_REQUIRE(d->precision == FQL_PRECISION_FP32, "fql_mlp_forward: FP32 only");
+  FQL_REQUIRE(d->precision == FQL_PRECISION_FP32 || d->precision == FQL_PRECISION_FP32_TC, "fql_mlp_forward: FP32 / FP32_TC only");
   const NetView& nv = L.net[net];
   FwdWs f;
   const size_t need = carve_forward(d, rows, nv.ens, nv.in_dim, nv.out_dim, nv.ln, nullptr, &f);

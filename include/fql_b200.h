@@ -38,8 +38,12 @@ enum { FQL_LEAF_KERNEL = 0, FQL_LEAF_BIAS = 1, FQL_LEAF_LN_SCALE = 2, FQL_LEAF_L
 /* Arithmetic mode of the contractions. */
 enum { FQL_PRECISION_FP32 = 0,      /* fp32 FFMA everywhere: parity mode (1e-5 vs the fp32/fp64 oracle)          */
        FQL_PRECISION_BF16_TC = 1,   /* bf16 operands on tcgen05, fp32 accumulate/epilogue, fp32 master weights   */
-       FQL_PRECISION_BF16_ENC = 2 };/* pixel configs: the ImpalaEncoders (89 % of the FLOPs) as bf16 implicit-GEMM
+       FQL_PRECISION_BF16_ENC = 2,  /* pixel configs: the ImpalaEncoders (89 % of the FLOPs) as bf16 implicit-GEMM
                                      * convolutions on tcgen05 (fp32 accumulate, bf16 activations), MLPs in fp32  */
+       FQL_PRECISION_FP32_TC = 3 }; /* the FP32 schedule with every Dense contraction on tcgen05 as 3xTF32: operands split into
+                                     * tf32 hi + lo, lo*hi + hi*lo + hi*hi into an fp32 accumulator (each product within ~2^-20
+                                     * relative); everything else fp32 as in FP32.  Same 1e-5 parity tolerance.  State
+                                     * observations only. */
 
 /* Static problem description: agents/fql.py:249-270 (get_config) + shapes fixed at create() (:192-194). */
 typedef struct FqlDims {
@@ -269,6 +273,23 @@ int fql_test_gelu_bwd_bf16(const float* dH, const float* Z, float* dZ, void* dZb
 /* column sums of bf16 X [G][M][N] (N % 64 == 0) ADDED into out[g0 * out_stride_g0 + g1 * out_stride_g1 + n], g = g1 * G0 + g0 */
 int fql_test_colsum_bf16(const void* X, int64_t G, int64_t M, int32_t N, float* out, int64_t out_stride_g0, int32_t G0,
                          int64_t out_stride_g1, void* stream);
+
+/* ---- test hook: the fp32 grouped GEMM of the MLP passes (launch_gemm, fql_b200/csrc/common.cuh GemmArgs) on caller buffers ------------
+ * C[M,N] = opA(A)[M,K] opB(B)[K,N] for the P x S x E groups g = (p * S + s) * E + e, operand X of group g at X.base[p] +
+ * s * X.stride_s + e * X.stride_e; epilogue in this order: + bias[N], out_pre = v, v *= gelu'(mulz), v = gelu(v) (act_gelu), out = v
+ * (bias / mulz / out_pre optional).  trans_a: A stored [K][M]; trans_b: B stored [N][K].  precision FQL_PRECISION_FP32 runs the FFMA
+ * kernel, FQL_PRECISION_FP32_TC the 3xTF32 tensor-core kernel; enqueue-only. */
+typedef struct FqlTestGPtr {
+  const void* base[3];
+  int64_t stride_s, stride_e;
+} FqlTestGPtr;
+typedef struct FqlTestGemmF32 {
+  int32_t M, N, K, P, S, E;
+  int32_t lda, ldb, ldo, ld_pre, ld_mulz;
+  int32_t trans_a, trans_b, act_gelu;
+  FqlTestGPtr A, B, bias, mulz, out_pre, out;
+} FqlTestGemmF32;
+int fql_test_gemm_f32(const FqlTestGemmF32* g, int32_t precision, void* stream);
 
 /* ---- test hooks: the tensor-core ImpalaEncoder of FQL_PRECISION_BF16_ENC / _TC (fql_b200/csrc/encoder_tc.cu) ------------------------
  * Each launches its kernels exactly as the encoder passes of the step do; nothing here is used by the step.  bf16 tensors are NHWC. */
