@@ -26,8 +26,9 @@ class FqlDims(C.Structure):
 
 
 class FqlHparams(C.Structure):
+    # per_seed: NULL, or a device array [num_seeds] of FqlHparams whose entry s holds lr / discount / tau / alpha / one_minus_tau of seed s
     _fields_ = [(n, C.c_float) for n in ('lr', 'beta1', 'beta2', 'eps', 'discount', 'tau', 'alpha', 'one_minus_beta1',
-                                         'one_minus_beta2', 'one_minus_tau')] + [('reserved', C.c_float * 2)]
+                                         'one_minus_beta2', 'one_minus_tau')] + [('per_seed', C.c_void_p)]
 
 
 class FqlLeaf(C.Structure):

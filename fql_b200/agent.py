@@ -27,10 +27,33 @@ INFO_KEYS = ('critic/critic_loss', 'critic/q_mean', 'critic/q_max', 'critic/q_mi
 NOISE_KEYS = ('z_next', 'x0', 't', 'z', 'z_metric')
 _BATCH_KEYS = ('observations', 'actions', 'next_observations', 'rewards', 'masks')
 _PIN_RING = 4   # pinned staging blocks per batch size
+# hyperparameters that may differ between the vectorised seeds (FqlHparams.per_seed); everything else is shared
+PER_SEED_KEYS = ('alpha', 'discount', 'tau', 'lr')
 
 
 def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
+
+
+def _check_per_seed(per_seed, num_seeds):
+    """{key: sequence of num_seeds values} -> {key: tuple of floats}, or None.  Raises ValueError on anything else."""
+    if per_seed is None:
+        return None
+    if not isinstance(per_seed, dict):
+        raise ValueError(f'per_seed must be a dict of per-seed sequences (got {type(per_seed).__name__})')
+    out = {}
+    for k, v in per_seed.items():
+        if k not in PER_SEED_KEYS:
+            raise ValueError(f'per_seed: {k!r} cannot vary per seed; the keys allowed are {PER_SEED_KEYS}.  Structural keys (network '
+                             f'shapes, layer_norm, actor_layer_norm, q_agg, normalize_q_loss, flow_steps, batch_size, encoder) are shared '
+                             f'by all seeds')
+        a = np.asarray(v, dtype=np.float64)
+        if a.shape != (num_seeds,):
+            raise ValueError(f'per_seed[{k!r}]: expected {num_seeds} values (one per seed), got shape {a.shape}')
+        if not np.isfinite(a).all():
+            raise ValueError(f'per_seed[{k!r}]: values must be finite (got {a.tolist()})')
+        out[k] = tuple(float(x) for x in a)
+    return out or None
 
 
 class LazyInfo(dict):
@@ -128,7 +151,10 @@ class FQLAgent:
     # ------------------------------------------------------------------ construction (agents/fql.py:173-246)
     @classmethod
     def create(cls, seed, ex_observations, ex_actions, config, *, num_seeds=1, device=None, precision='fp32',
-               process_group=None, world_size=None, rank=None):
+               process_group=None, world_size=None, rank=None, per_seed=None):
+        """per_seed: hyperparameter sweeps as vectorised seeds -- a dict from a subset of PER_SEED_KEYS ('alpha', 'discount', 'tau',
+        'lr') to sequences of num_seeds values; seed i trains with those values (seed_config(i)), every other key of `config` is
+        shared.  The table goes to the device once and every entry point of the step reads it."""
         self = cls.__new__(cls)
         cfg = dict(config)
         ex_observations = np.asarray(ex_observations)
@@ -148,6 +174,7 @@ class FQLAgent:
         self.config = cfg
         self.device = torch.device(device if device is not None else f'cuda:{torch.cuda.current_device()}')
         self.num_seeds = int(num_seeds)
+        self._per_seed = _check_per_seed(per_seed, self.num_seeds)
         self.pg = process_group
         self.world = 1
         if process_group is not None:
@@ -172,6 +199,13 @@ class FQLAgent:
             _lib.check(self._lib.fql_context_create(C.byref(ctx)), 'fql_context_create')
         self._ctx = ctx
         self._hp = _lib.make_hparams(lr=cfg['lr'], discount=cfg['discount'], tau=cfg['tau'], alpha=cfg['alpha'])
+        self._hp_table = None
+        if self._per_seed is not None:
+            # one FqlHparams per seed (make_hparams: 1 - tau in double, as for the shared struct), one host-to-device copy
+            rows = [_lib.make_hparams(**{k: self.seed_config(i)[k] for k in PER_SEED_KEYS}) for i in range(self.num_seeds)]
+            host = (_lib.FqlHparams * self.num_seeds)(*rows)
+            self._hp_table = torch.frombuffer(bytearray(host), dtype=torch.uint8).to(self.device)
+            self._hp.per_seed = self._hp_table.data_ptr()
         self._dims_cache = {}
         d = self._dims(int(cfg.get('batch_size', 256)))
         self._leaves, self._arena = _lib.layout(d)
@@ -211,6 +245,20 @@ class FQLAgent:
         self.rng = ss.generate_state(2, dtype=np.uint32)
         self.network = TrainStateView(self)
         return self
+
+    @property
+    def per_seed(self):
+        """The per-seed hyperparameters given to create ({key: tuple of num_seeds floats}), or None when all seeds share `config`."""
+        return None if self._per_seed is None else dict(self._per_seed)
+
+    def seed_config(self, i):
+        """The config agent (seed) i trains with: `config` with its per-seed values."""
+        if not 0 <= i < self.num_seeds:
+            raise IndexError(f'seed {i} out of range for {self.num_seeds} seeds')
+        cfg = dict(self.config)
+        for k, v in (self._per_seed or {}).items():
+            cfg[k] = v[i]
+        return cfg
 
     def _attach_peer_memory(self, d, group):
         """Data parallel over NVLink peer memory (include/fql_b200.h, fql_dp_attach): the gradient arena, the metric gather buffer and

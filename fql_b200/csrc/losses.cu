@@ -131,6 +131,7 @@ __device__ float dp_sum_over_ranks(const DpLamArgs& l, int s, int S, float mine)
   return tot;
 }
 
+template <bool TABLE>
 __global__ void critic_post_kernel(StepShape sh, FqlHparams hp, FqlBatch b, WsPtrs w, float* raw, int parts, DpLamArgs dpl) {
   // grid (S, nc): CTA c of seed s reduces rows c, c + nc, ... ; the partial sums of the nc CTAs are combined in CTA order by the
   // last one to finish (ticket counter), so the result does not depend on scheduling
@@ -142,12 +143,13 @@ __global__ void critic_post_kernel(StepShape sh, FqlHparams hp, FqlBatch b, WsPt
   const float* q_c = w.C_out + ((int64_t)(1 * S + s) * 2) * B;
   const float* q_p = w.C_out + ((int64_t)(2 * S + s) * 2) * B;
   const float inv_2gb = 1.0f / (2.0f * (float)sh.GB);
+  const float discount = seed_hp<TABLE>(hp, s, &FqlHparams::discount);
   float sq = 0.f, qs = 0.f, qmx = -INFINITY, qmn = INFINITY, ps = 0.f, pa = 0.f;
   for (int r = cta * blockDim.x + threadIdx.x; r < B; r += nc * blockDim.x) {
     if (parts & 1) {
       const float t0 = q_t[r], t1 = q_t[B + r];
       const float nq = sh.q_agg_min ? fminf(t0, t1) : (t0 + t1) * 0.5f;
-      const float y = b.rewards[(int64_t)s * B + r] + hp.discount * b.masks[(int64_t)s * B + r] * nq;
+      const float y = b.rewards[(int64_t)s * B + r] + discount * b.masks[(int64_t)s * B + r] * nq;
 #pragma unroll
       for (int h = 0; h < 2; h++) {
         const float q = q_c[h * B + r];
@@ -256,12 +258,13 @@ __global__ void euler_update_kernel(StepShape sh, WsPtrs w, int step) {
 
 // Distillation loss + dL/da_pi (fql.py:65-79): da = alpha*2(a_pi-target)/(GB*A) + [dQ/da through clip].
 // dX0: [S][2][B][KC] input-gradient of the critic(s, clip a_pi) pass; the two heads are summed (input broadcast).
+template <bool TABLE>
 __global__ void actor_grad_kernel(StepShape sh, FqlHparams hp, WsPtrs w, float* raw, __nv_bfloat16* dapib) {
   __shared__ float red[32];
   const int s = blockIdx.x;
   const int A = sh.A, B = sh.B, KC = sh.F + sh.A;
   const float* api = w.O_out + ((int64_t)s * 3 * B + B) * A;
-  const float scale = hp.alpha * 2.0f / ((float)sh.GB * (float)A);
+  const float scale = seed_hp<TABLE>(hp, s, &FqlHparams::alpha) * 2.0f / ((float)sh.GB * (float)A);
   float sq = 0.f;
   // dapib (tensor-core mode): the same gradient as the zero-padded bf16 [B][64] operand of the first dgrad GEMM
   if (dapib) {
@@ -286,11 +289,12 @@ __global__ void actor_grad_kernel(StepShape sh, FqlHparams hp, WsPtrs w, float* 
 }
 
 // info[13] from the (all-reduced) raw accumulators + gradient statistics.
+template <bool TABLE>
 __global__ void finalize_info_kernel(StepShape sh, FqlHparams hp, const float* raw, int ranks, const float* gstats, float* info,
                                      int with_grad_stats) {
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= sh.S) return;
-  fql_finalize_info_seed(sh, hp, raw, ranks, gstats, info, s, with_grad_stats);
+  fql_finalize_info_seed<TABLE>(sh, hp, raw, ranks, gstats, info, s, with_grad_stats);
 }
 
 // clip(x) elementwise (fql.py:152)
@@ -349,7 +353,7 @@ int launch_critic_post(const StepShape& sh, const FqlHparams& hp, const FqlBatch
   if (dpl) l = *dpl;
   int nc = (sh.B + 2047) / 2048;
   nc = nc < 1 ? 1 : (nc > 64 ? 64 : nc);
-  critic_post_kernel<<<dim3(sh.S, nc), 1024, 0, st>>>(sh, hp, b, w, raw, parts, l);
+  (hp.per_seed ? critic_post_kernel<true> : critic_post_kernel<false>)<<<dim3(sh.S, nc), 1024, 0, st>>>(sh, hp, b, w, raw, parts, l);
   FQL_CHECK_LAUNCH();
   return 0;
 }
@@ -365,13 +369,15 @@ int launch_euler_update(const StepShape& sh, const WsPtrs& w, int step, cudaStre
   return 0;
 }
 int launch_actor_grad(const StepShape& sh, const FqlHparams& hp, const WsPtrs& w, float* raw, cudaStream_t st, void* dapib) {
-  actor_grad_kernel<<<dim3(sh.S, loss_ctas(sh)), 1024, 0, st>>>(sh, hp, w, raw, reinterpret_cast<__nv_bfloat16*>(dapib));
+  (hp.per_seed ? actor_grad_kernel<true> : actor_grad_kernel<false>)<<<dim3(sh.S, loss_ctas(sh)), 1024, 0, st>>>(
+      sh, hp, w, raw, reinterpret_cast<__nv_bfloat16*>(dapib));
   FQL_CHECK_LAUNCH();
   return 0;
 }
 int launch_finalize_info(const StepShape& sh, const FqlHparams& hp, const float* raw, int ranks, const float* gstats, float* info,
                          int with_grad_stats, cudaStream_t st) {
-  finalize_info_kernel<<<(sh.S + 63) / 64, 64, 0, st>>>(sh, hp, raw, ranks, gstats, info, with_grad_stats);
+  (hp.per_seed ? finalize_info_kernel<true> : finalize_info_kernel<false>)<<<(sh.S + 63) / 64, 64, 0, st>>>(sh, hp, raw, ranks, gstats, info,
+                                                                                                      with_grad_stats);
   FQL_CHECK_LAUNCH();
   return 0;
 }

@@ -14,6 +14,7 @@ namespace {
 // ADAM_U consecutive blocks per CTA, all loads issued before the first use.  Measured on B200 (110 MB pass, cold L2): U = 1
 // 21.8 us, U = 4 27.3 us (registers halve the resident CTAs) -- more CTAs beat more loads per thread.
 constexpr int ADAM_U = 1;
+template <bool TABLE>
 __global__ void __launch_bounds__(256) adam_polyak_stats_kernel(Layout L, FqlHparams hp, float* __restrict__ params,
                                                                 float* __restrict__ mu, float* __restrict__ nu,
                                                                 const float* __restrict__ grads,
@@ -43,6 +44,8 @@ __global__ void __launch_bounds__(256) adam_polyak_stats_kernel(Layout L, FqlHpa
   // optax bias_correction: 1 - decay**count in float32, correctly rounded -- computed once per step by zero_bc_kernel (a double
   // pow in every CTA of this pass cost ~3 us per CTA wave)
   const float bc1 = bc[0], bc2 = bc[1];
+  const float lr = seed_hp<TABLE>(hp, s, &FqlHparams::lr), tau = seed_hp<TABLE>(hp, s, &FqlHparams::tau),
+              omt = seed_hp<TABLE>(hp, s, &FqlHparams::one_minus_tau);
   __shared__ float smx[ADAM_U][8], smn[ADAM_U][8], ssq[ADAM_U][8];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
 #pragma unroll
@@ -63,7 +66,7 @@ __global__ void __launch_bounds__(256) adam_polyak_stats_kernel(Layout L, FqlHpa
       vr[i] = hp.beta2 * vr[i] + hp.one_minus_beta2 * gi * gi;
       const float mhat = mr[i] / bc1;
       const float vhat = vr[i] / bc2;
-      pn[i] = pr[i] + (-hp.lr * (mhat / (sqrtf(vhat) + hp.eps)));
+      pn[i] = pr[i] + (-lr * (mhat / (sqrtf(vhat) + hp.eps)));
     }
     *reinterpret_cast<float4*>(params + base + off) = make_float4(pn[0], pn[1], pn[2], pn[3]);
     if (shadow) {  // bf16 tensor-core operand copy of the fresh parameters (same [in,out] layout)
@@ -75,11 +78,10 @@ __global__ void __launch_bounds__(256) adam_polyak_stats_kernel(Layout L, FqlHpa
     if (pol[u]) {  // Polyak with the pre-step critic values still in registers
       const int64_t toff = base + off - cri.begin + tgt.begin;
       float4 t4 = tp[u];
-      const float omt = hp.one_minus_tau;
-      t4.x = pr[0] * hp.tau + t4.x * omt;
-      t4.y = pr[1] * hp.tau + t4.y * omt;
-      t4.z = pr[2] * hp.tau + t4.z * omt;
-      t4.w = pr[3] * hp.tau + t4.w * omt;
+      t4.x = pr[0] * tau + t4.x * omt;
+      t4.y = pr[1] * tau + t4.y * omt;
+      t4.z = pr[2] * tau + t4.z * omt;
+      t4.w = pr[3] * tau + t4.w * omt;
       *reinterpret_cast<float4*>(params + toff) = t4;
       if (shadow) {
         __nv_bfloat162 lo = __floats2bfloat162_rn(t4.x, t4.y), hi = __floats2bfloat162_rn(t4.z, t4.w);
@@ -110,6 +112,7 @@ __global__ void __launch_bounds__(256) adam_polyak_stats_kernel(Layout L, FqlHpa
 
 // one CTA per seed, one WARP per leaf (lanes stride over the leaf's block partials): per-leaf L2 norms, then the three
 // scalars of flax_utils.py:147-149
+template <bool TABLE>
 __global__ void __launch_bounds__(1024) grad_stats_final_kernel(Layout L, const float* __restrict__ partials,
                                                                 float* __restrict__ gstats, int32_t* count_inc, FinArgs fin) {
   const int s = blockIdx.x;
@@ -150,7 +153,7 @@ __global__ void __launch_bounds__(1024) grad_stats_final_kernel(Layout L, const 
     gstats[s * 4 + 1] = b;
     gstats[s * 4 + 2] = c;
     if (s == 0 && count_inc) count_inc[0] += 1;  // optax count / TrainState.step advance (flax_utils.py:126)
-    if (fin.info) fql_finalize_info_seed(fin.sh, fin.hp, fin.raw, fin.ranks, gstats, fin.info, s, 1);
+    if (fin.info) fql_finalize_info_seed<TABLE>(fin.sh, fin.hp, fin.raw, fin.ranks, gstats, fin.info, s, 1);
   }
 }
 
@@ -169,11 +172,13 @@ __global__ void zero_bc_kernel(float4* p, int64_t n4, const int32_t* __restrict_
 }
 
 // FQLAgent.target_update (agents/fql.py:113-120) on its own: target <- tau * critic + (1 - tau) * target, plus the bf16 shadow.
+template <bool TABLE>
 __global__ void target_update_kernel(float* __restrict__ params, __nv_bfloat16* __restrict__ shadow, int64_t arena, int64_t shadow_seed,
-                                     int64_t cri0, int64_t tgt0, int64_t n, float tau, float omt) {
+                                     int64_t cri0, int64_t tgt0, int64_t n, FqlHparams hp) {
   const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 4;
   const int s = blockIdx.y;
   if (i >= n) return;
+  const float tau = seed_hp<TABLE>(hp, s, &FqlHparams::tau), omt = seed_hp<TABLE>(hp, s, &FqlHparams::one_minus_tau);
   const float4 p = *reinterpret_cast<const float4*>(params + s * arena + cri0 + i);
   float4 t = *reinterpret_cast<const float4*>(params + s * arena + tgt0 + i);
   t.x = p.x * tau + t.x * omt;
@@ -201,7 +206,7 @@ int launch_adam_polyak_stats(const Layout& L, const FqlHparams& hp, int S, float
   if (blk1 < 0) blk1 = nblk;
   if (blk1 <= blk0) return 0;
   dim3 grid((blk1 - blk0 + ADAM_U - 1) / ADAM_U, S);
-  adam_polyak_stats_kernel<<<grid, 256, 0, st>>>(L, hp, params, mu, nu, grads, bc, partials, reinterpret_cast<__nv_bfloat16*>(shadow), shadow_seed, blk0, blk1,
+  (hp.per_seed ? adam_polyak_stats_kernel<true> : adam_polyak_stats_kernel<false>)<<<grid, 256, 0, st>>>(L, hp, params, mu, nu, grads, bc, partials, reinterpret_cast<__nv_bfloat16*>(shadow), shadow_seed, blk0, blk1,
                                                  nblk);
   FQL_CHECK_LAUNCH();
   return 0;
@@ -212,7 +217,7 @@ int launch_grad_stats_final(const Layout& L, int S, const float* partials, float
   FinArgs f;
   memset(&f, 0, sizeof(f));
   if (fin) f = *fin;
-  grad_stats_final_kernel<<<S, 1024, 0, st>>>(L, partials, gstats, count_inc, f);
+  (f.hp.per_seed ? grad_stats_final_kernel<true> : grad_stats_final_kernel<false>)<<<S, 1024, 0, st>>>(L, partials, gstats, count_inc, f);
   FQL_CHECK_LAUNCH();
   return 0;
 }
@@ -230,6 +235,7 @@ extern "C" int fql_target_update(const FqlDims* d, const FqlHparams* hp, float* 
   Layout L;
   FQL_TRY(fql_build_layout(d, &L));
   FQL_REQUIRE(hp && params, "fql_target_update: NULL argument");
+  FQL_TRY(check_seed_table(hp));
   const NetView& cri = L.net[FQL_NET_CRITIC];
   const NetView& tgt = L.net[FQL_NET_TARGET_CRITIC];
   const int64_t n = cri.end - cri.begin;
@@ -237,9 +243,9 @@ extern "C" int fql_target_update(const FqlDims* d, const FqlHparams* hp, float* 
   const bool tcm = d->precision == FQL_PRECISION_BF16_TC;
   FQL_REQUIRE(!tcm || shadow, "FQL_PRECISION_BF16_TC needs the bf16 shadow");
   dim3 grid((unsigned)((n / 4 + 255) / 256), d->num_seeds);
-  target_update_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+  (hp->per_seed ? target_update_kernel<true> : target_update_kernel<false>)<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
       params, tcm ? reinterpret_cast<__nv_bfloat16*>(shadow) : nullptr, L.arena, tcm ? tc_shadow_seed_elems(d, L) : 0, cri.begin, tgt.begin, n,
-      hp->tau, hp->one_minus_tau);
+      *hp);
   FQL_CHECK_LAUNCH();
   if (tcm) FQL_TRY(tc_refresh_shadow_lastlayer(d, L, params, shadow, reinterpret_cast<cudaStream_t>(stream)));
   return 0;

@@ -1258,6 +1258,7 @@ int run_step_on(FqlContext* ctx, const StepCall& c, cudaStream_t S0) {
 int run_step(FqlContext* ctx, const StepCall& c, void* stream) {
   FQL_REQUIRE(ctx != nullptr, "context is NULL");
   FQL_REQUIRE(c.d && c.hp && c.st, "NULL argument");
+  FQL_TRY(check_seed_table(c.hp));
   cudaStream_t user = reinterpret_cast<cudaStream_t>(stream);
   if (user != nullptr && user != cudaStreamLegacy) return run_step_on(ctx, c, user);
   FQL_CHECK_CUDA(cudaEventRecord(ctx->ev[6], user));
@@ -1269,6 +1270,17 @@ int run_step(FqlContext* ctx, const StepCall& c, void* stream) {
 }
 
 }  // namespace
+
+int check_seed_table(const FqlHparams* hp) {
+  if (!hp->per_seed) return 0;
+  FQL_REQUIRE(((uintptr_t)hp->per_seed & (alignof(FqlHparams) - 1)) == 0, "FqlHparams.per_seed must be %zu-byte aligned",
+              alignof(FqlHparams));
+  cudaPointerAttributes a;
+  FQL_CHECK_CUDA(cudaPointerGetAttributes(&a, hp->per_seed));
+  FQL_REQUIRE(a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged,
+              "FqlHparams.per_seed must point to device memory (one FqlHparams per seed)");
+  return 0;
+}
 
 extern "C" int fql_update_step(FqlContext* ctx, const FqlDims* d, const FqlHparams* hp, const FqlBatch* batch,
                                const FqlState* st, float* info, void* workspace, size_t ws_bytes, void* stream) {

@@ -101,8 +101,18 @@ int launch_grad_stats_final(const Layout& L, int S, const float* partials, float
                             const FinArgs* fin = nullptr);
 
 #ifdef __CUDACC__
+// Hyper-parameter `f` (lr, discount, tau, alpha, one_minus_tau) of seed s: entry s of the per-seed table (FqlHparams.per_seed) in
+// the TABLE instantiation of a kernel, else the shared value.  The launchers pick the instantiation on the host, so a step without a
+// table runs the same code as before tables existed.
+template <bool TABLE>
+__device__ __forceinline__ float seed_hp(const FqlHparams& hp, int s, float FqlHparams::*f) {
+  if constexpr (TABLE) return hp.per_seed[s].*f;
+  else return hp.*f;
+}
+
 // info[13] of one seed from the (all-gathered) raw accumulators + gradient statistics (agents/fql.py:38-44, 78-90, flax_utils.py:147-149).
 // data parallel: `raw` is the all-gather of every rank's accumulators [ranks][S][FQL_NUM_RAW]: sums add, max / -min take the max
+template <bool TABLE>
 __device__ __forceinline__ void fql_finalize_info_seed(const StepShape& sh, const FqlHparams& hp, const float* raw, int ranks, const float* gstats,
                                                        float* info, int s, int with_grad_stats) {
   float rw[FQL_NUM_RAW];
@@ -125,7 +135,7 @@ __device__ __forceinline__ void fql_finalize_info_seed(const StepShape& sh, cons
   o[1] = rw[RAW_Q_SUM] / (2.0f * gb);
   o[2] = rw[RAW_Q_MAX];
   o[3] = -rw[RAW_Q_NEGMIN];
-  o[4] = bc + hp.alpha * distill + q_loss;
+  o[4] = bc + seed_hp<TABLE>(hp, s, &FqlHparams::alpha) * distill + q_loss;
   o[5] = bc;
   o[6] = distill;
   o[7] = q_loss;
@@ -140,6 +150,8 @@ __device__ __forceinline__ void fql_finalize_info_seed(const StepShape& sh, cons
   }
 }
 #endif
+// FqlHparams.per_seed, when set, must be device (or managed) memory: a host array would fault inside the step.
+int check_seed_table(const FqlHparams* hp);
 int launch_zero(float* p, int64_t n, cudaStream_t st);
 // zero p[0..n) and (count != NULL) write optax's float32 bias corrections {1 - b1^(count+1), 1 - b2^(count+1)} to bc[0..1]
 int launch_zero_bc(float* p, int64_t n, const int32_t* count, const FqlHparams& hp, float* bc, cudaStream_t st, int* tickets = nullptr,

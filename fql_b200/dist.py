@@ -56,3 +56,17 @@ def shard_seeds(num_seeds: int, rank: int, world: int) -> range:
         raise ValueError(f'{num_seeds} seeds do not divide over {world} ranks')
     per = num_seeds // world
     return range(rank * per, (rank + 1) * per)
+
+
+def shard_per_seed(per_seed, rank: int, world: int):
+    """FQLAgent.create(per_seed=...) of rank r under seed sharding: every sequence sliced to the seeds shard_seeds gives the rank, so
+    each rank's agents train with their own hyperparameters.  None stays None."""
+    if per_seed is None:
+        return None
+    lengths = {len(v) for v in per_seed.values()}
+    if len(lengths) > 1:
+        raise ValueError(f'per_seed sequences differ in length: { {k: len(v) for k, v in per_seed.items()} }')
+    if not lengths:
+        return {}
+    r = shard_seeds(lengths.pop(), rank, world)
+    return {k: list(v)[r.start:r.stop] for k, v in per_seed.items()}

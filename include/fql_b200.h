@@ -65,14 +65,22 @@ typedef struct FqlDims {
                               * {0,0,0} = state-based */
 } FqlDims;
 
-/* Hyper-parameters that are runtime scalars. agents/fql.py:255-264, optax.adam defaults. */
+/* Hyper-parameters that are runtime scalars. agents/fql.py:255-264, optax.adam defaults.  48 bytes, 8-byte aligned (per_seed).
+ *
+ * Hyper-parameter sweeps: with per_seed != NULL the num_seeds vectorised agents train with their own lr, discount, tau and alpha
+ * (an alpha grid x seeds in one step).  Each kernel that reads one of them reads it once per CTA (or per seed) from the table,
+ * indexed by its seed.  beta1 / beta2 / eps stay shared: the Adam bias correction is computed once per step.  Everything that
+ * fixes a shape or a code path is in FqlDims and is shared by all seeds.  The table is read when the step runs, so a captured
+ * step graph sees its current contents; a different table pointer is a different argument set (another graph). */
 typedef struct FqlHparams {
   float lr, beta1, beta2, eps;
   float discount, tau, alpha;
   /* (1-beta1), (1-beta2), (1-tau) evaluated in double on the host and then rounded, as the reference's Python-float
-   * arithmetic does (optax `(1 - decay) * g`, fql.py:116 `tp * (1 - tau)`): 1.0f-0.999f differs from (float)0.001 by 1.3e-5. */
+   * arithmetic does (optax `(1 - decay) * g`, fql.py:116 `tp * (1 - tau)`): 1.0f-0.999f differs from (float)0.001 by 1.3e-5.
+   * A per-seed table carries one_minus_tau per entry for the same reason. */
   float one_minus_beta1, one_minus_beta2, one_minus_tau;
-  float reserved[2];
+  const struct FqlHparams* per_seed; /* NULL: every seed uses this struct.  Else: device array [num_seeds]; entry s supplies
+                                      * lr, discount, tau, alpha, one_minus_tau of seed s (its other fields are ignored) */
 } FqlHparams;
 
 typedef struct FqlLeaf {
@@ -193,7 +201,8 @@ int fql_compute_flow_actions(FqlContext* ctx, const FqlDims* d, const float* par
 int fql_mlp_forward(FqlContext* ctx, const FqlDims* d, int32_t net, const float* params, const float* x, float* y,
                     int32_t rows, void* workspace, size_t ws_bytes, void* stream);
 /* FQLAgent.target_update(network, 'critic') (agents/fql.py:113-120) on its own: target_critic <- tau * critic + (1 - tau) * target_critic
- * in place in the parameter arena (fql_update_step already contains it, fused into the optimizer pass). */
+ * in place in the parameter arena (fql_update_step already contains it, fused into the optimizer pass); tau and 1 - tau per seed
+ * when hp->per_seed is set. */
 int fql_target_update(const FqlDims* d, const FqlHparams* hp, float* params, void* shadow, void* stream);
 /* Rebuild the bf16 operand shadow from fp32 params (after create()/restore; the step keeps it current itself). */
 int fql_refresh_shadow(const FqlDims* d, const float* params, void* shadow, void* stream);
